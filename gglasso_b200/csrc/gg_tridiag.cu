@@ -44,7 +44,7 @@ struct TrWs {
     double* y;       // (M,n)
     int* cnt;        // (M) tile arrival counters of tr_step_kernel (zero between launches)
 #ifdef TR_TIMING
-    long long* dbg;  // (n,2,8) time stamps of one CTA per launch (instrumented build only)
+    long long* dbg;  // (n,2,8) time stamps of one CTA per launch (instrumented build only; nullptr: no stamps)
 #endif
 };
 
@@ -55,7 +55,7 @@ __device__ __forceinline__ long long tr_now()
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
     return t;
 }
-#define TR_STAMP(kind, slot) do { if (tr_stamp_on) ws.dbg[((size_t)j * 2 + (kind)) * 8 + (slot)] = tr_now(); } while (0)
+#define TR_STAMP(kind, slot) do { if (tr_stamp_on && ws.dbg) ws.dbg[((size_t)j * 2 + (kind)) * 8 + (slot)] = tr_now(); } while (0)
 #else
 #define TR_STAMP(kind, slot) do { } while (0)
 #endif
@@ -1706,6 +1706,88 @@ static int dbg_nonfinite(const double* dptr, int M, int n, int ncheck, cudaStrea
     return 0;
 }
 
+// Side streams for work forked off the caller's stream.  They and their events belong to the calling host thread and
+// the current device (thread_local, created on first use), so concurrent solves on other host threads never share a
+// stream or an event with this one.  Fork and join are event record / wait only, which is legal inside stream capture.
+#define GG_SIDE_MAX 3
+struct GgSides {
+    cudaStream_t s[GG_SIDE_MAX];
+    cudaEvent_t fork, join[GG_SIDE_MAX];
+};
+
+static GgSides* gg_sides()          // nullptr if they cannot be created
+{
+    static thread_local GgSides tl[64] = {};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
+    GgSides& g = tl[dev];
+    if (!g.fork && cudaEventCreateWithFlags(&g.fork, cudaEventDisableTiming) != cudaSuccess) {
+        g.fork = nullptr;
+        return nullptr;
+    }
+    for (int i = 0; i < GG_SIDE_MAX; ++i) {
+        if (!g.s[i] && cudaStreamCreateWithFlags(&g.s[i], cudaStreamNonBlocking) != cudaSuccess) {
+            g.s[i] = nullptr;
+            return nullptr;
+        }
+        if (!g.join[i] && cudaEventCreateWithFlags(&g.join[i], cudaEventDisableTiming) != cudaSuccess) {
+            g.join[i] = nullptr;
+            return nullptr;
+        }
+    }
+    return &g;
+}
+
+// side streams 0..k-1 wait for the work issued to s so far
+static int gg_fork(const GgSides& g, cudaStream_t s, int k)
+{
+    cudaError_t e = cudaEventRecord(g.fork, s);
+    for (int i = 0; i < k && e == cudaSuccess; ++i) e = cudaStreamWaitEvent(g.s[i], g.fork, 0);
+    return (int)e;
+}
+
+// s waits for the work issued to side streams 0..k-1 so far (all k are joined even if one fails)
+static int gg_join(const GgSides& g, cudaStream_t s, int k)
+{
+    cudaError_t r = cudaSuccess;
+    for (int i = 0; i < k; ++i) {
+        cudaError_t e = cudaEventRecord(g.join[i], g.s[i]);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(s, g.join[i], 0);
+        if (r == cudaSuccess) r = e;
+    }
+    return (int)r;
+}
+
+// stage-1 workspace of matrices m0.. of the batch (every array has the matrix index outermost)
+static TrWs tr_ws_from(const TrWs& tw, int m0, int n)
+{
+    const size_t nn = (size_t)n * n, mn = (size_t)m0 * n;
+    TrWs t = tw;
+    t.Vh += m0 * nn;
+    t.tau += mn;
+    t.d += mn;
+    t.e += mn;
+    t.vbuf += 2 * mn;
+    t.w += TR_QMAX * mn;
+    t.y += mn;
+    t.cnt += m0;
+#ifdef TR_TIMING
+    if (m0) t.dbg = nullptr;         // only the chain that holds matrix 0 stamps
+#endif
+    return t;
+}
+
+// Concurrent chains of stage 1 (see gg_eigh_tridiag_impl): TR_GROUPS chains while the batch's upper triangles
+// (4 M t^2 bytes) exceed TR_SPLIT_MB.  Measured on B200 (profiles/r03_tr_groups.json): two groups beat three and four,
+// and 12 MB beats 6 / 24 / 48 MB (a lower threshold splits K=3 p=1000 and K=10 p=500, which then get slower).
+#ifndef TR_GROUPS
+#define TR_GROUPS 2
+#endif
+#ifndef TR_SPLIT_MB
+#define TR_SPLIT_MB 12
+#endif
+static_assert(TR_GROUPS >= 1 && TR_GROUPS <= GG_SIDE_MAX + 1, "TR_GROUPS chains need TR_GROUPS - 1 side streams");
+
 // write-back depth of the tridiagonalisation (see TR_QMAX): env GG_TR_LAZY in [1, TR_QMAX], default 3
 int gg_tr_lazy_depth()
 {
@@ -1895,30 +1977,97 @@ int gg_eigh_tridiag_impl(double* A, double* D, int M, int n, const double* ctrl,
                 if (write) kb = j;
             }
         }
-        for (int j = jb; j < js && chain && !merged; ++j) {
+        // Attributes of a chain launch: programmatic dependence on the stream's previous kernel unless `dep` is false
+        // (the first launch after a fork or a join, which must wait for the event in full); with `prio` the greatest
+        // scheduling priority (see the concurrent chains below).
+        int prio_lo = 0, prio_hi = 0;
+        cudaLaunchAttribute ca[2];
+        auto chain_cfg = [&](cudaStream_t st, bool dep, bool prio) {
+            cfg.stream = st;
+            cfg.attrs = ca;
+            cfg.numAttrs = 0;
+            if (dep && !no_pdl) {
+                ca[cfg.numAttrs].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+                ca[cfg.numAttrs++].val.programmaticStreamSerializationAllowed = 1;
+            }
+            if (prio) {
+                ca[cfg.numAttrs].id = cudaLaunchAttributePriority;
+                ca[cfg.numAttrs++].val.priority = prio_hi;
+            }
+        };
+        // column step j and trailing-matrix pass j over the Mb matrices of (Ab, twb, skb), on stream st
+        auto column = [&](double* Ab, const TrWs& twb, const int* skb, int Mb, cudaStream_t st, bool dep, bool prio,
+                          int j, int write) -> int {
             if (which != 2) {
                 const int len = n - j;
                 const int thr = len <= 2048 ? 256 : 512;
-                cfg.gridDim = dim3(M); cfg.blockDim = dim3(thr); cfg.dynamicSmemBytes = 0;
+                chain_cfg(st, dep, prio);
+                cfg.gridDim = dim3(Mb); cfg.blockDim = dim3(thr); cfg.dynamicSmemBytes = 0;
                 cudaError_t e;
                 gg_count_launch(1);
-                if (len <= 512) e = cudaLaunchKernelEx(&cfg, tr_col_kernel<2, 256, true>, (const double*)A, n, j, kb, tw, (const int*)skip);
-                else if (len <= 1024) e = cudaLaunchKernelEx(&cfg, tr_col_kernel<4, 256, true>, (const double*)A, n, j, kb, tw, (const int*)skip);
-                else if (len <= 2048) e = cudaLaunchKernelEx(&cfg, tr_col_kernel<8, 256, true>, (const double*)A, n, j, kb, tw, (const int*)skip);
-                else if (len <= 8192) e = cudaLaunchKernelEx(&cfg, tr_col_kernel<16, 512, false>, (const double*)A, n, j, kb, tw, (const int*)skip);
+                if (len <= 512) e = cudaLaunchKernelEx(&cfg, tr_col_kernel<2, 256, true>, (const double*)Ab, n, j, kb, twb, skb);
+                else if (len <= 1024) e = cudaLaunchKernelEx(&cfg, tr_col_kernel<4, 256, true>, (const double*)Ab, n, j, kb, twb, skb);
+                else if (len <= 2048) e = cudaLaunchKernelEx(&cfg, tr_col_kernel<8, 256, true>, (const double*)Ab, n, j, kb, twb, skb);
+                else if (len <= 8192) e = cudaLaunchKernelEx(&cfg, tr_col_kernel<16, 512, false>, (const double*)Ab, n, j, kb, twb, skb);
                 else return -5;
                 if (e != cudaSuccess) return (int)e;
+                dep = true;
             }
-            // write pass: the pending list is full, or the tail kernel takes over next (it expects only pair js-1)
-            const int write = (j - kb >= lazy_q || (j == js - 1 && j > kb)) ? 1 : 0;
             if (j < n - 1 && which != 1) {
                 const int t = n - j - 1;
                 const int nt = (t + SV_T - 1) / SV_T;
-                cfg.gridDim = dim3(nt * (nt + 1) / 2, M); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = 0;
+                chain_cfg(st, dep, false);
+                cfg.gridDim = dim3(nt * (nt + 1) / 2, Mb); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = 0;
                 gg_count_launch(1);
-                cudaError_t e = cudaLaunchKernelEx(&cfg, tr_symv_kernel, A, n, j, kb, write, tw, (const int*)skip, nt);
+                cudaError_t e = cudaLaunchKernelEx(&cfg, tr_symv_kernel, Ab, n, j, kb, write, twb, skb, nt);
                 if (e != cudaSuccess) return (int)e;
             }
+            return 0;
+        };
+        // write pass: the pending list is full, or the tail kernel takes over next (it expects only pair js-1)
+        auto write_pass = [&](int j) { return (j - kb >= lazy_q || (j == js - 1 && j > kb)) ? 1 : 0; };
+
+        // Columns [jb, jg): concurrent chains.  The chain is serial only within a matrix (y_j -> v_j -> y_{j+1}), so
+        // while the trailing blocks are large the batch runs as G chains over contiguous groups of matrices, group g
+        // on side stream g-1 (group 0 on s): one chain's column step and launch boundaries overlap another's
+        // trailing-matrix pass, whose tiles also fill the last, partial wave of the other grids.  Launches are issued
+        // column-major, so every chain is at the same column with the same write-back schedule kb, and the chains
+        // rejoin at column jg to go on as one chain over the batch: short columns cannot afford G times the host
+        // time of their launches (about 2 us each).  The column steps run at the greatest scheduling priority: they
+        // are on their chain's critical path, and their CTAs must not queue behind the pending tiles of another
+        // chain's pass (measured at K=20, p=1000 with a 24 MB threshold: gg_eigh 15.19 ms with, 15.86 ms without).
+        const int G = M < TR_GROUPS ? M : TR_GROUPS;
+        int jg = jb;
+        GgSides* sides = nullptr;
+        if (chain && !merged && !use_blocked && G > 1) {
+            while (jg < js && 4.0 * M * (double)(n - jg - 1) * (n - jg - 1) > TR_SPLIT_MB * 1048576.0) ++jg;
+            if (jg > jb && (!(sides = gg_sides()) || gg_fork(*sides, s, G - 1) != 0)) jg = jb;
+            if (jg > jb) cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
+        }
+        bool dep = true;                  // the next launch on s may depend programmatically on its predecessor
+        if (jg > jb) {
+            TrWs twg[TR_GROUPS];
+            for (int g = 0; g < G; ++g) twg[g] = tr_ws_from(tw, g * M / G, n);
+            int rc = 0;
+            for (int j = jb; j < jg && rc == 0; ++j) {
+                const int write = write_pass(j);
+                for (int g = 0; g < G && rc == 0; ++g) {
+                    const int m0 = g * M / G, m1 = (g + 1) * M / G;
+                    rc = column(A + m0 * nn, twg[g], skip + m0, m1 - m0, g ? sides->s[g - 1] : s, j > jb, true, j,
+                                write);
+                }
+                if (write) kb = j;
+            }
+            const int rj = gg_join(*sides, s, G - 1);
+            if (rc != 0) return rc;
+            if (rj != 0) return rj;
+            dep = false;
+        }
+        for (int j = jg; j < js && chain && !merged; ++j) {
+            const int write = write_pass(j);
+            const int rc = column(A, tw, skip, M, s, dep, false, j, write);
+            if (rc != 0) return rc;
+            dep = true;
             if (write) kb = j;
         }
         if (js < n && !(use_blocked && prof12)) {
@@ -1926,6 +2075,7 @@ int gg_eigh_tridiag_impl(double* A, double* D, int M, int n, const double* ctrl,
             const size_t tsm = sizeof(double) * ((size_t)ts * (ts | 1) + 3 * ts + 64 + 4);
             cudaFuncSetAttribute(tr_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,       // (per device)
                                  (int)(sizeof(double) * ((size_t)TR_TAIL * (TR_TAIL | 1) + 3 * TR_TAIL + 68)));
+            chain_cfg(s, dep, false);
             cfg.gridDim = dim3(M); cfg.blockDim = dim3(512); cfg.dynamicSmemBytes = tsm;
             gg_count_launch(1);
             cudaError_t e = cudaLaunchKernelEx(&cfg, tr_tail_kernel, (const double*)A, n, js, tw, (const int*)skip, chain ? 1 : 0);
@@ -1955,29 +2105,15 @@ int gg_eigh_tridiag_impl(double* A, double* D, int M, int n, const double* ctrl,
     cudaFuncSetAttribute(bb_x_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,                  // (per device)
                          (int)(sizeof(double) * (BB_NB * (BB_NB + 1) + BB_GTRI)));
     const bool use_big = npanels > 0 && which != 4 && bt_big && n >= BB_MIN;
-    // GG_BT_SIDE=1: the three preparation launches run on a side stream next to stage 2 (fork after stage 1, join
-    // before stage 3).  The side stream belongs to the calling host thread and device (thread_local), the two events
-    // to this call: nothing is shared between concurrent solves.
-    cudaEvent_t ev_join = nullptr;
+    // GG_BT_SIDE=1: the three preparation launches run on side stream 0 of the calling thread (gg_sides) next to
+    // stage 2 (fork after stage 1, join before stage 3): nothing is shared between concurrent solves.
+    GgSides* bt_side = nullptr;
     if (use_big) {
         cudaStream_t ps = s;
-        if (sytrd_blocked_env("GG_BT_SIDE", 0)) {
-            static thread_local cudaStream_t tl_side[64] = {};
-            int dev = 0;
-            cudaGetDevice(&dev);
-            if (dev >= 0 && dev < 64) {
-                if (!tl_side[dev] && cudaStreamCreateWithFlags(&tl_side[dev], cudaStreamNonBlocking) != cudaSuccess)
-                    tl_side[dev] = nullptr;
-                cudaEvent_t ev_fork = nullptr;
-                if (tl_side[dev] && cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming) == cudaSuccess &&
-                    cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming) == cudaSuccess) {
-                    cudaEventRecord(ev_fork, s);
-                    cudaStreamWaitEvent(tl_side[dev], ev_fork, 0);
-                    ps = tl_side[dev];
-                } else ev_join = nullptr;
-                if (ev_fork) cudaEventDestroy(ev_fork);      // (released once the pending work has used it)
-            }
-        }
+        if (sytrd_blocked_env("GG_BT_SIDE", 0) && (bt_side = gg_sides()) && gg_fork(*bt_side, s, 1) == 0)
+            ps = bt_side->s[0];
+        else
+            bt_side = nullptr;
         const int nt64 = (n + BB_T - 1) / BB_T;
         gg_count_launch(1);
         bb_gram_kernel<<<dim3(BB_NB / BB_T, BB_NB / BB_T, M * npb), 256, 0, ps>>>(tw.Vh, n, npb, Gb, skip);
@@ -1986,7 +2122,6 @@ int gg_eigh_tridiag_impl(double* A, double* D, int M, int n, const double* ctrl,
         gg_count_launch(1);
         bb_vprime_kernel<<<dim3(nt64, BB_NB / BB_T, M * npb), 256, 0, ps>>>(tw.Vh, Xb, n, npb, Vp, skip);
         GG_CHECK_LAUNCH();
-        if (ps != s) cudaEventRecord(ev_join, ps);
     }
 
     // ---- stage 2 ----
@@ -2037,10 +2172,7 @@ int gg_eigh_tridiag_impl(double* A, double* D, int M, int n, const double* ctrl,
     // eigenvalues of the root are in lam[0]; eigenvectors of T (rows) in A
     gg_count_launch(1);
     dc_unscale_kernel<<<dim3(4, M), 256, 0, s>>>(dw.lam[0], scale, n, D, skip);
-    if (ev_join) {
-        cudaStreamWaitEvent(s, ev_join, 0);
-        cudaEventDestroy(ev_join);
-    }
+    if (bt_side) gg_join(*bt_side, s, 1);
     if (stop_after == 2) return 0;
 
     // ---- stage 3 ----
