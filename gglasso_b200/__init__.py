@@ -1,8 +1,8 @@
 """gglasso_b200 -- B200 (sm_100a) implementation of GGLasso's ADMM hot path.
 
 Drop-in replacements for ``gglasso.solver.admm_solver.ADMM_MGL``,
-``gglasso.solver.single_admm_solver.ADMM_SGL`` and ``block_SGL`` (same call signatures and return
-dicts), backed by hand-written CUDA kernels behind a C ABI (include/gglasso_b200.h).
+``gglasso.solver.single_admm_solver.ADMM_SGL`` and ``block_SGL``, and of the second-order solvers
+``gglasso.solver.ppdna_solver.PPDNA`` / ``warmPPDNA`` (same call signatures and return dicts), backed by hand-written CUDA kernels behind a C ABI (include/gglasso_b200.h).
 ``install()`` rebinds those names inside an importable ``gglasso`` package so that
 ``glasso_problem`` and ``grid_search`` run unmodified on top of the GPU path.
 """
@@ -10,6 +10,7 @@ from .solver.admm_solver import ADMM_MGL  # noqa: F401
 from .solver.single_admm_solver import ADMM_SGL, block_SGL, get_connected_components  # noqa: F401
 from .solver.functional_sgl_admm import ADMM_FSGL  # noqa: F401
 from .solver.ext_admm_solver import ext_ADMM_MGL  # noqa: F401
+from .solver.ppdna_solver import PPDNA, warmPPDNA  # noqa: F401
 from ._lib import GGLassoB200Error, LIB_PATH  # noqa: F401
 
 __version__ = "0.1.0"
@@ -30,7 +31,7 @@ def install():
         "gglasso.problem": {"ADMM_MGL": ADMM_MGL, "ADMM_SGL": ADMM_SGL, "block_SGL": block_SGL,
                             "ext_ADMM_MGL": ext_ADMM_MGL},
         "gglasso.helper.model_selection": {"ADMM_SGL": ADMM_SGL, "block_SGL": block_SGL},
-        "gglasso.solver.ppdna_solver": {"ADMM_MGL": ADMM_MGL},
+        "gglasso.solver.ppdna_solver": {"ADMM_MGL": ADMM_MGL, "PPDNA": PPDNA, "warmPPDNA": warmPPDNA},
         "gglasso.solver.functional_sgl_admm": {"ADMM_FSGL": ADMM_FSGL},
         "gglasso.solver.ext_admm_solver": {"ext_ADMM_MGL": ext_ADMM_MGL},
     }

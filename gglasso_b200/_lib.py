@@ -56,6 +56,16 @@ SIGNATURES = {
     "gg_asym_max": (_i, [_vp, _i, _i, _vp, _vp]),
     "gg_gershgorin_min": (_i, [_vp, _i, _i, _vp, _sz, _vp, _vp]),
     "gg_host_tv1d": (None, [ctypes.POINTER(_d), _i, _i, _d]),
+    "gg_ppdna_build": (_i, [_vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "gg_ppdna_spectral": (_i, [_vp, _vp, _d, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "gg_ppdna_nparts": (_i, [_i]),
+    "gg_ppdna_prox": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _d, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "gg_ppdna_jp_nparts": (_i, [_i]),
+    "gg_ppdna_jp": (_i, [_vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "gg_ppdna_hess": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "gg_ppdna_cg_init": (_i, [_vp, _i, _i, _d, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "gg_ppdna_cg": (_i, [_i, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                         _vp]),
 }
 
 _LIB = None

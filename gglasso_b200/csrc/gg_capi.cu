@@ -49,6 +49,23 @@ size_t gg_tridiag_ws_bytes(int, int);
 int gg_sytrd_phase_times(unsigned long long*);
 int gg_tr_lazy_depth();
 int gg_gershgorin_min_impl(const double*, int, int, void*, size_t, double*, cudaStream_t);
+int gg_launch_ppdna_build(const double*, const double*, const double*, const double*, const double*, double, double, int,
+                          int, double*, double*, double*, const double*, cudaStream_t);
+int gg_launch_ppdna_spectral(const double*, const double*, double, int, int, double*, double*, double*, double*,
+                             const double*, cudaStream_t);
+int gg_launch_ppdna_prox(const double*, const double*, const double*, const double*, const double*, const double*, double,
+                         double, double, int, int, int, double*, double*, unsigned char*, double*, double*,
+                         const double*, cudaStream_t);
+int gg_launch_ppdna_jp(const double*, const double*, const unsigned char*, const double*, const double*, double, double,
+                       int, int, int, double*, double*, const double*, cudaStream_t);
+int gg_launch_ppdna_hess(const double*, const double*, const double*, const double*, const double*, const unsigned char*,
+                         const double*, double, double, int, int, int, double*, double*, double*, double*,
+                         const double*, cudaStream_t);
+int gg_launch_ppdna_cg_init(const double*, int, int, double, int, double*, double*, double*, double*, double*,
+                            cudaStream_t);
+int gg_launch_ppdna_cg(int, const double*, const double*, const double*, const double*, const unsigned char*,
+                       const double*, double, double, int, int, int, double*, double*, double*, double*, double*,
+                       double*, double*, double*, cudaStream_t);
 
 #include <atomic>
 static std::atomic<long long> g_launches{0};
@@ -254,5 +271,64 @@ int gg_gershgorin_min(const double* A, int M, int p, void* ws, size_t ws_bytes, 
 }
 
 void gg_host_tv1d(double* v, int n, int stride, double lam) { gg_tv1d_inplace(v, n, stride, lam); }
+
+int gg_ppdna_build(const double* Omega_t, const double* Theta_t, const double* S, const double* X, const double* dX,
+                   double s, double sigma, int K, int p, double* Xs, double* W, double* V, const double* flag,
+                   void* stream)
+{
+    if (K <= 0 || p <= 0 || !(sigma > 0.0)) return -1;
+    return gg_launch_ppdna_build(Omega_t, Theta_t, S, X, dX, s, sigma, K, p, Xs, W, V, flag, (cudaStream_t)stream);
+}
+
+int gg_ppdna_spectral(const double* Vt, const double* D, double sigma, int K, int p, double* Q, double* phi,
+                      double* logdet, double* Omega, const double* flag, void* stream)
+{
+    if (K <= 0 || p <= 0 || !(sigma > 0.0)) return -1;
+    return gg_launch_ppdna_spectral(Vt, D, sigma, K, p, Q, phi, logdet, Omega, flag, (cudaStream_t)stream);
+}
+
+int gg_ppdna_prox(const double* V, const double* Omega, const double* Omega_t, const double* Theta_t, const double* X,
+                  const double* S, double lambda1, double lambda2, double sigma, int reg, int K, int p, double* Theta,
+                  double* G, unsigned char* code, double* jscale, double* partials, const double* flag, void* stream)
+{
+    if (K <= 0 || p <= 0 || reg < 0 || reg > 1 || !(sigma > 0.0) || partials == nullptr) return -1;
+    return gg_launch_ppdna_prox(V, Omega, Omega_t, Theta_t, X, S, lambda1, lambda2, sigma, reg, K, p, Theta, G, code,
+                                jscale, partials, flag, (cudaStream_t)stream);
+}
+
+int gg_ppdna_jp(const double* Din, const double* V, const unsigned char* code, const double* jscale, const double* Jphi,
+                double sigma, double lambda1, int reg, int K, int p, double* Out, double* partials, const double* flag,
+                void* stream)
+{
+    if (K <= 0 || p <= 0 || reg < 0 || reg > 1) return -1;
+    return gg_launch_ppdna_jp(Din, V, code, jscale, Jphi, sigma, lambda1, reg, K, p, Out, partials, flag,
+                              (cudaStream_t)stream);
+}
+
+int gg_ppdna_hess(const double* Vt, const double* Q, const double* phi, const double* Din, const double* V,
+                  const unsigned char* code, const double* jscale, double sigma, double lambda1, int reg, int K, int p,
+                  double* Y, double* Z, double* Out, double* partials, const double* flag, void* stream)
+{
+    if (K <= 0 || p <= 0 || reg < 0 || reg > 1 || !(sigma > 0.0) || Out == Din) return -1;
+    return gg_launch_ppdna_hess(Vt, Q, phi, Din, V, code, jscale, sigma, lambda1, reg, K, p, Y, Z, Out, partials, flag,
+                                (cudaStream_t)stream);
+}
+
+int gg_ppdna_cg_init(const double* G, int K, int p, double tol, int max_iter, double* d, double* r, double* pv,
+                     double* cg, double* partials, void* stream)
+{
+    if (K <= 0 || p <= 0) return -1;
+    return gg_launch_ppdna_cg_init(G, K, p, tol, max_iter, d, r, pv, cg, partials, (cudaStream_t)stream);
+}
+
+int gg_ppdna_cg(int iters, const double* Vt, const double* Q, const double* phi, const double* V,
+                const unsigned char* code, const double* jscale, double sigma, double lambda1, int reg, int K, int p,
+                double* d, double* r, double* pv, double* q, double* Y, double* Z, double* cg, double* partials,
+                void* stream)
+{
+    if (iters < 0 || K <= 0 || p <= 0 || reg < 0 || reg > 1 || !(sigma > 0.0)) return -1;
+    return gg_launch_ppdna_cg(iters, Vt, Q, phi, V, code, jscale, sigma, lambda1, reg, K, p, d, r, pv, q, Y, Z, cg,
+                              partials, (cudaStream_t)stream);
+}
 
 }  // extern "C"

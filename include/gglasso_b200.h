@@ -196,6 +196,48 @@ int gg_asym_max(const double* A, int M, int p, double* out, void* stream);
  * ws: at least the gg_eigh workspace of the same (M,p). */
 int gg_gershgorin_min(const double* A, int M, int p, void* ws, size_t ws_bytes, double* out, void* stream);
 
+/* PPDNA, the proximal point dual Newton method for GGL / FGL (src/gglasso/solver/ppdna_solver.py PPA_subproblem:65,
+ * PPDNA:160; ggl_helper.py:74-159,218-249,323-437).  One problem of K instances (K <= 90); X is the UNSCALED dual;
+ * flag (device double, may be NULL): every kernel is a no-op once *flag != 0.
+ *  gg_ppdna_build   : Xs = X + s dX (dX may be NULL), W = Omega_t - sigma (S + Xs), V = Theta_t + sigma Xs, full
+ *                     matrices (replaces the W / V assembly of PPA_subproblem, ppdna_solver.py:88-100)
+ *  gg_ppdna_spectral: from gg_eigh's Vt and eigenvalues D of W: Q = Vt^T, phi = phi+(D, sigma) (K,p), logdet[k] =
+ *                     sum log phi, Omega = Vt^T diag(phi) Vt   (phiplus, ggl_helper.py:272-303)
+ *  gg_ppdna_prox    : Theta = prox_p(V, sigma lambda1, sigma lambda2) (same device routines as gg_prox_mgl), G =
+ *                     Theta - Omega, the Jacobian data of prox_p (code: (K,p,p) bytes, jscale: (p,p) doubles) and
+ *                     gg_ppdna_nparts(p) x 6 partial sums {<S,Omega>, P(Theta), <X,Omega-Theta>, |Omega-Omega_t|^2,
+ *                     |Theta-Theta_t|^2, |G|^2}; the caller zeroes partials once (eval_jacobian_prox_p,
+ *                     ggl_helper.py:218-252; Phi_t, :357)
+ *  gg_ppdna_jp      : Out = sigma (Jphi + J_P(V)[Din]) (Jphi may be NULL or alias Out); partials (may be NULL):
+ *                     gg_ppdna_jp_nparts(p) values of <Din, Out>   (jacobian_prox_phi_*, ggl_helper.py:74-159)
+ *  gg_ppdna_hess    : Out = sigma (Q (Gamma o (Q^T Din Q)) Q^T + J_P(V)[Din]), Gamma_ab = phi_a phi_b/(phi_a phi_b +
+ *                     sigma), on FP64 tensor cores; Y, Z: (K,p,p) scratch   (hessian_Y, ggl_helper.py:361-370)
+ *  gg_ppdna_cg_init : d = 0, r = pv = -G, CG state cg (8 doubles) armed with tol and the iteration cap
+ *  gg_ppdna_cg      : enqueues `iters` CG iterations on H d = -G (no-ops once cg[3] != 0); cg[0] = |r|^2, cg[4] =
+ *                     iterations done   (cg_ppdna, ggl_helper.py:372-409).  partials: at least 1184 doubles. */
+int gg_ppdna_build(const double* Omega_t, const double* Theta_t, const double* S, const double* X, const double* dX,
+                   double s, double sigma, int K, int p, double* Xs, double* W, double* V, const double* flag,
+                   void* stream);
+int gg_ppdna_spectral(const double* Vt, const double* D, double sigma, int K, int p, double* Q, double* phi,
+                      double* logdet, double* Omega, const double* flag, void* stream);
+int gg_ppdna_nparts(int p);
+int gg_ppdna_prox(const double* V, const double* Omega, const double* Omega_t, const double* Theta_t, const double* X,
+                  const double* S, double lambda1, double lambda2, double sigma, int reg, int K, int p, double* Theta,
+                  double* G, unsigned char* code, double* jscale, double* partials, const double* flag, void* stream);
+int gg_ppdna_jp_nparts(int p);
+int gg_ppdna_jp(const double* Din, const double* V, const unsigned char* code, const double* jscale, const double* Jphi,
+                double sigma, double lambda1, int reg, int K, int p, double* Out, double* partials, const double* flag,
+                void* stream);
+int gg_ppdna_hess(const double* Vt, const double* Q, const double* phi, const double* Din, const double* V,
+                  const unsigned char* code, const double* jscale, double sigma, double lambda1, int reg, int K, int p,
+                  double* Y, double* Z, double* Out, double* partials, const double* flag, void* stream);
+int gg_ppdna_cg_init(const double* G, int K, int p, double tol, int max_iter, double* d, double* r, double* pv,
+                     double* cg, double* partials, void* stream);
+int gg_ppdna_cg(int iters, const double* Vt, const double* Q, const double* phi, const double* V,
+                const unsigned char* code, const double* jscale, double sigma, double lambda1, int reg, int K, int p,
+                double* d, double* r, double* pv, double* q, double* Y, double* Z, double* cg, double* partials,
+                void* stream);
+
 /* Host-side execution of the exact device TV-prox routine (unit tests without a GPU). */
 void gg_host_tv1d(double* v, int n, int stride, double lam);
 
