@@ -5,8 +5,10 @@ Drop-in replacements for ``gglasso.solver.admm_solver.ADMM_MGL``,
 ``gglasso.solver.ppdna_solver.PPDNA`` / ``warmPPDNA`` (same call signatures and return dicts), backed by hand-written CUDA kernels behind a C ABI (include/gglasso_b200.h).
 ``install()`` rebinds those names inside an importable ``gglasso`` package so that
 ``glasso_problem`` and ``grid_search`` run unmodified on top of the GPU path.
+``ADMM_MGL_batch`` (no counterpart in the reference, so ``install()`` leaves it alone) solves many MGL problems of the
+same shape in one device loop.
 """
-from .solver.admm_solver import ADMM_MGL  # noqa: F401
+from .solver.admm_solver import ADMM_MGL, ADMM_MGL_batch  # noqa: F401
 from .solver.single_admm_solver import ADMM_SGL, block_SGL, get_connected_components  # noqa: F401
 from .solver.functional_sgl_admm import ADMM_FSGL  # noqa: F401
 from .solver.ext_admm_solver import ext_ADMM_MGL  # noqa: F401

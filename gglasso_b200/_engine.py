@@ -306,8 +306,8 @@ class AdmmState:
     def omega_step(self, upper=False):
         lib, st = self.lib, self.stream
         if upper:       # upper triangles only (see run_admm): the tridiagonal eigensolver reads nothing else of W
-            _lib.check(lib.gg_build_w_upper(_p(self.Theta), _p(self.X), _p(self.S), _p(self.nk), _p(self.ctrl),
-                                            self.M, self.p, _p(self.W), st), "gg_build_w_upper")
+            _lib.check(lib.gg_build_w_upper_batch(_p(self.Theta), _p(self.X), _p(self.S), _p(self.nk), _p(self.ctrl),
+                                                  self.mpp, self.p, self.nprob, _p(self.W), st), "gg_build_w_upper")
         else:
             _lib.check(lib.gg_build_w(_p(self.Theta), _p(self.L), _p(self.X), _p(self.S), _p(self.nk), _p(self.ctrl),
                                       self.M, self.p, self.mpp, _p(self.W), st), "gg_build_w")
@@ -344,10 +344,12 @@ class AdmmState:
         _lib.check(self.lib.gg_scale_pending(_p(self.X), _p(self.ctrl), self.M, self.p, self.mpp, self.stream),
                    "gg_scale_pending")
 
-    def asym_max(self, A):
+    def asym_max(self, A, per_problem=False):
         n = self.lib.gg_sgl_nparts(self.p, self.M)
         out = torch.empty((self.M, n), dtype=torch.float64, device=self.dev)
         _lib.check(self.lib.gg_asym_max(_p(A), self.M, self.p, _p(out), self.stream), "gg_asym_max")
+        if per_problem:
+            return out.reshape(self.nprob, -1).amax(dim=1).cpu().numpy()
         return float(out.max().item())
 
     def is_posdef(self, A, res=None):
@@ -390,6 +392,19 @@ class AdmmState:
         D = self.eig.eigh(B, ctrl=None, mpp=1, vectors=0, stream=self.stream)
         return D.min()
 
+    def min_eig_per_problem(self, A):
+        """smallest eigenvalue of each problem's matrices in A, or -- where the Gershgorin bound of all of them is
+        positive -- that bound (a certificate of positive definiteness, like is_posdef); device tensor (nprob,).
+        The eigendecomposition of the stack is enqueued only when some problem is not certified."""
+        g = torch.empty(self.M, dtype=torch.float64, device=self.dev)
+        _lib.check(self.lib.gg_gershgorin_min(_p(A), self.M, self.p, _p(self.eig.ws), self.eig.ws_bytes, _p(g),
+                                              self.stream), "gg_gershgorin_min")
+        g = g.reshape(self.nprob, -1).amin(dim=1)
+        if bool((g > 0.0).all().item()):
+            return g
+        D = self.eig.eigh(A.clone(), ctrl=None, mpp=1, vectors=0, stream=self.stream)
+        return torch.where(g > 0.0, g, D.reshape(self.nprob, -1).amin(dim=1))
+
     def mark(self):
         """event on the main stream: everything enqueued so far (the ADMM loop) -- used as the dependency of the
         overlapped D2H so that it does not wait for work enqueued later (the PD-check eigendecomposition)."""
@@ -420,8 +435,12 @@ class AdmmState:
 def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None, lam_mat=None, rho=1.0,
              max_iter=1000, tol=1e-7, rtol=1e-4, stopping_criterion="boyd", update_rho=True, verbose=False,
              measure=False, latent=False, mu=None, nk=None, header=None, check_every=None, trace=None,
-             check_symmetric=False, pvec=None, Mblk=None, print_rho=False, state=None, graph=None):
+             check_symmetric=False, pvec=None, Mblk=None, print_rho=False, state=None, graph=None, K=None):
     """Run the device ADMM loop.  ``kind``: 'mgl' (one problem of K matrices) or 'sgl' (M problems).
+
+    ``K`` ('mgl' only): matrices per problem.  The stacks then hold M/K independent MGL problems (ADMM_MGL_batch),
+    problem q owning matrices q*K .. q*K+K-1 and control block q; ``lambda1`` / ``lambda2`` may be arrays of one value
+    per problem.  Default: one problem of all M matrices.
 
     ``state``: an AdmmState of the same shapes from an earlier call (lambda grids): its buffers, workspace and captured
     iteration graphs are reused.  ``graph``: run the iterations as replays of two captured CUDA graphs (one per
@@ -432,7 +451,12 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
     """
     S3 = S if S.ndim == 3 else S[None]       # numpy arrays or device tensors
     M, p, _ = S3.shape
-    mpp = M if kind == "mgl" else 1
+    mpp = (M if K is None else K) if kind == "mgl" else 1
+    if kind == "mgl" and M // mpp > 1:
+        if measure or stopping_criterion != "boyd":
+            raise NotImplementedError("a batch of MGL problems supports stopping_criterion='boyd' without measure only")
+        if mpp > K_TILE_MAX:
+            raise NotImplementedError(f"a batch of MGL problems needs K <= {K_TILE_MAX} (tile-pair prox), got K = {mpp}")
     if state is not None:
         st = state
         assert st.M == M and st.p == p and st.mpp == mpp and st.latent == latent and st.hist_cap >= max_iter
@@ -445,8 +469,14 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
                        None if X_0 is None else X_0.reshape(S3.shape), mpp, rho, max_iter, latent, nk=nk, mu=mu,
                        lam_mat=lam_mat, pvec=pvec)
         if kind == "mgl":                        # lambdas live in the control block (see GG_C_LAM1)
-            st.ctrl[:, C_LAM1] = lambda1
-            st.ctrl[:, C_LAM2] = lambda2
+            if np.ndim(lambda1) == 0 and np.ndim(lambda2) == 0:
+                st.ctrl[:, C_LAM1] = lambda1
+                st.ctrl[:, C_LAM2] = lambda2
+            else:                                # one value per problem of a batch
+                lam = np.broadcast_to(np.stack(np.broadcast_arrays(np.asarray(lambda1, dtype=np.float64),
+                                                                   np.asarray(lambda2, dtype=np.float64)), -1),
+                                      (st.nprob, 2))
+                st.ctrl[:, C_LAM1:C_LAM2 + 1] = torch.from_numpy(np.array(lam)).to(st.dev)
     lib, stream = st.lib, st.stream
     nprob = st.nprob
     regi = {"GGL": 0, "FGL": 1}.get(reg, -1)
@@ -459,11 +489,14 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
         nparts_fused = nt * nt
     else:
         nparts_fused = lib.gg_sgl_nparts(p, M)
-    prox_mgl_fn = lib.gg_prox_mgl
+    prox_mgl_fn = lib.gg_prox_mgl_batch
     nparts_dual = lib.gg_sgl_nparts(p, M) * mpp
     # K beyond the shared-memory layout of the fused tile-pair prox (K x 272 doubles per CTA): the row-band prox of the
     # K-sharded path takes over on one device (pack -> band prox -> unpack fused with the dual update)
-    big_K = kind == "mgl" and M > K_TILE_MAX
+    big_K = kind == "mgl" and mpp > K_TILE_MAX
+    # scalar lambdas of the kernel arguments; the MGL kernels read each problem's lambdas from its control block
+    if kind == "mgl":
+        lam1_arg, lam2_arg = float(np.ravel(lambda1)[0]), float(np.ravel(lambda2)[0])
     # Non-latent MGL on the tridiagonal eigensolver path: the iterations keep only the UPPER triangles of Theta, X and W
     # current (every consumer inside the loop reads nothing else; half the elementwise HBM traffic) and the lower
     # triangles are filled once after the loop -- prox_p's mirroring (ggl_helper.py:198-205) done once.
@@ -511,8 +544,9 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
         st.omega_step(upper)
         Cq = st.W if latent else None
         if upper:
-            _lib.check(lib.gg_prox_mgl_upper(_p(st.Omega_new), _p(st.Omega), _p(st.X), _p(st.Theta), _p(st.ctrl),
-                                             lambda1, lambda2, regi, M, p, _p(partials), sm), "gg_prox_mgl_upper")
+            _lib.check(lib.gg_prox_mgl_upper_batch(_p(st.Omega_new), _p(st.Omega), _p(st.X), _p(st.Theta),
+                                                   _p(st.ctrl), lam1_arg, lam2_arg, regi, mpp, p, nprob, _p(partials),
+                                                   sm), "gg_prox_mgl_upper")
         elif big_K:
             _lib.check(lib.gg_pack_bands(_p(st.Omega_new), _p(st.L), _p(st.X), _p(st.ctrl), M, p, 1, _p(vband), sm),
                        "gg_pack_bands")
@@ -522,7 +556,8 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
                                           _p(st.ctrl), M, p, 1, _p(partials), sm), "gg_unpack_dual")
         elif kind == "mgl":
             _lib.check(prox_mgl_fn(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(Cq),
-                                   _p(st.ctrl), lambda1, lambda2, regi, M, p, _p(partials), sm), "gg_prox_mgl")
+                                   _p(st.ctrl), lam1_arg, lam2_arg, regi, mpp, p, nprob, _p(partials), sm),
+                       "gg_prox_mgl")
         elif Mblk is not None:
             _lib.check(lib.gg_prox_fsgl(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(Cq),
                                         _p(st.ctrl), float(lambda1), int(Mblk), M, p, _p(partials), _p(blk_nrm), sm),
@@ -607,8 +642,9 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
             logdet_dev = torch.log(0.5 * (torch.sqrt(Dw * Dw + 4 * beta[:, None]) + Dw)).sum()
         C = st.W if latent else None
         if upper:
-            _lib.check(lib.gg_prox_mgl_upper(_p(st.Omega_new), _p(st.Omega), _p(st.X), _p(st.Theta), _p(st.ctrl),
-                                             lambda1, lambda2, regi, M, p, _p(partials), stream), "gg_prox_mgl_upper")
+            _lib.check(lib.gg_prox_mgl_upper_batch(_p(st.Omega_new), _p(st.Omega), _p(st.X), _p(st.Theta),
+                                                   _p(st.ctrl), lam1_arg, lam2_arg, regi, mpp, p, nprob, _p(partials),
+                                                   stream), "gg_prox_mgl_upper")
         elif big_K:
             _lib.check(lib.gg_pack_bands(_p(st.Omega_new), _p(st.L), _p(st.X), _p(st.ctrl), M, p, 1, _p(vband), stream),
                        "gg_pack_bands")
@@ -618,7 +654,7 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
                                           _p(st.ctrl), M, p, 1, _p(partials), stream), "gg_unpack_dual")
         elif kind == "mgl":
             _lib.check(prox_mgl_fn(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(C),
-                                   _p(st.ctrl), lambda1, lambda2, regi, M, p, _p(partials), stream),
+                                   _p(st.ctrl), lam1_arg, lam2_arg, regi, mpp, p, nprob, _p(partials), stream),
                        "gg_prox_mgl")
         elif Mblk is not None:
             _lib.check(lib.gg_prox_fsgl(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(C),

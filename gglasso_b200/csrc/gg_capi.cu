@@ -10,11 +10,11 @@ int gg_launch_prox_sgl(const double*, const double*, const double*, double*, dou
 int gg_launch_dual_update(double*, const double*, const double*, const double*, const double*, const double*, int,
                           int, int, int, double*, cudaStream_t);
 int gg_launch_prox_mgl(const double*, const double*, const double*, double*, double*, double*, const double*, double,
-                       double, int, int, int, double*, cudaStream_t);
+                       double, int, int, int, int, double*, cudaStream_t);
 int gg_launch_prox_mgl_upper(const double*, const double*, double*, double*, const double*, double, double, int, int,
-                             int, double*, cudaStream_t);
-int gg_launch_build_w_upper(const double*, double*, const double*, const double*, const double*, int, int, double*,
-                            cudaStream_t);
+                             int, int, double*, cudaStream_t);
+int gg_launch_build_w_upper(const double*, double*, const double*, const double*, const double*, int, int, int,
+                            double*, cudaStream_t);
 int gg_launch_mirror_upper(double*, double*, int, int, cudaStream_t);
 int gg_launch_stop_update(const double*, int, double*, double*, int, const double*, double, double, int, int,
                           cudaStream_t);
@@ -138,7 +138,16 @@ int gg_prox_mgl(const double* Omega, const double* Omega_prev, const double* L, 
                 void* stream)
 {
     if (K <= 0 || p <= 0 || reg < 0 || reg > 1) return -1;
-    return gg_launch_prox_mgl(Omega, Omega_prev, L, X, Theta, C, ctrl, lambda1, lambda2, reg, K, p, partials,
+    return gg_launch_prox_mgl(Omega, Omega_prev, L, X, Theta, C, ctrl, lambda1, lambda2, reg, K, p, 1, partials,
+                              (cudaStream_t)stream);
+}
+
+int gg_prox_mgl_batch(const double* Omega, const double* Omega_prev, const double* L, double* X, double* Theta,
+                      double* C, const double* ctrl, double lambda1, double lambda2, int reg, int K, int p, int nprob,
+                      double* partials, void* stream)
+{
+    if (K <= 0 || p <= 0 || nprob <= 0 || nprob > 65535 || reg < 0 || reg > 1 || ctrl == nullptr) return -1;
+    return gg_launch_prox_mgl(Omega, Omega_prev, L, X, Theta, C, ctrl, lambda1, lambda2, reg, K, p, nprob, partials,
                               (cudaStream_t)stream);
 }
 
@@ -146,7 +155,16 @@ int gg_prox_mgl_upper(const double* Omega, const double* Omega_prev, double* X, 
                       double lambda1, double lambda2, int reg, int K, int p, double* partials, void* stream)
 {
     if (K <= 0 || p <= 0 || reg < 0 || reg > 1) return -1;
-    return gg_launch_prox_mgl_upper(Omega, Omega_prev, X, Theta, ctrl, lambda1, lambda2, reg, K, p, partials,
+    return gg_launch_prox_mgl_upper(Omega, Omega_prev, X, Theta, ctrl, lambda1, lambda2, reg, K, p, 1, partials,
+                                    (cudaStream_t)stream);
+}
+
+int gg_prox_mgl_upper_batch(const double* Omega, const double* Omega_prev, double* X, double* Theta, const double* ctrl,
+                            double lambda1, double lambda2, int reg, int K, int p, int nprob, double* partials,
+                            void* stream)
+{
+    if (K <= 0 || p <= 0 || nprob <= 0 || nprob > 65535 || reg < 0 || reg > 1 || ctrl == nullptr) return -1;
+    return gg_launch_prox_mgl_upper(Omega, Omega_prev, X, Theta, ctrl, lambda1, lambda2, reg, K, p, nprob, partials,
                                     (cudaStream_t)stream);
 }
 
@@ -154,7 +172,14 @@ int gg_build_w_upper(const double* Theta, double* X, const double* S, const doub
                      int p, double* W, void* stream)
 {
     if (K <= 0 || p <= 0) return -1;
-    return gg_launch_build_w_upper(Theta, X, S, nk, ctrl, K, p, W, (cudaStream_t)stream);
+    return gg_launch_build_w_upper(Theta, X, S, nk, ctrl, K, p, 1, W, (cudaStream_t)stream);
+}
+
+int gg_build_w_upper_batch(const double* Theta, double* X, const double* S, const double* nk, const double* ctrl, int K,
+                           int p, int nprob, double* W, void* stream)
+{
+    if (K <= 0 || K > 65535 || p <= 0 || nprob <= 0 || nprob > 65535 || ctrl == nullptr) return -1;
+    return gg_launch_build_w_upper(Theta, X, S, nk, ctrl, K, p, nprob, W, (cudaStream_t)stream);
 }
 
 int gg_mirror_upper(double* A0, double* A1, int M, int p, void* stream)

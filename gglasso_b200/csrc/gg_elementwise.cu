@@ -222,6 +222,16 @@ dual_update_kernel(double* __restrict__ X, const double* __restrict__ Omega, con
 #define PLD 17
 #define PSLOT (PT * PLD)   // 272
 
+// blockIdx.y read afresh at every use: the batched MGL kernels form the offset of problem q from it after the register-
+// heavy K-vector prox instead of keeping a 64-bit offset live across it (which costs registers / spills at the kernels'
+// launch bounds)
+__device__ __forceinline__ size_t gg_batch_offset(int K, int p)
+{
+    unsigned q;
+    asm volatile("mov.u32 %0, %%ctaid.y;" : "=r"(q));
+    return (size_t)q * K * ((size_t)p * p);
+}
+
 template <int REG, bool LATENT>
 __global__ void __launch_bounds__(PT * PT)
 prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Omega_prev,
@@ -242,9 +252,12 @@ prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Ome
     const int SJ = SI + sp;
     const int I = 4 * SI + ((blockIdx.x >> 2) & 3), J = 4 * SJ + (blockIdx.x & 3);
     if (I > J || J >= nt) return;
-    if (ctrl[GG_C_DONE] != 0.0) return;
-    const double inv_rho = 1.0 / ctrl[GG_C_RHO];
-    if (ctrl[GG_C_LAM1] > 0.0) { lambda1 = ctrl[GG_C_LAM1]; lambda2 = ctrl[GG_C_LAM2]; }
+    // problem q = blockIdx.y of a batch: control block q, matrices q*K.. (offset qo, folded into the element
+    // index so that the array arguments stay kernel parameters) and nt*nt partial sums
+    const double* cq = ctrl + (size_t)blockIdx.y * GG_CTRL_STRIDE;
+    if (cq[GG_C_DONE] != 0.0) return;
+    const double inv_rho = 1.0 / cq[GG_C_RHO];
+    if (cq[GG_C_LAM1] > 0.0) { lambda1 = cq[GG_C_LAM1]; lambda2 = cq[GG_C_LAM2]; }
     const double l1 = inv_rho * lambda1, l2 = inv_rho * lambda2;
     const int tr = threadIdx.x / PT, tc = threadIdx.x % PT;
     const size_t pp = (size_t)p * p;
@@ -255,7 +268,7 @@ prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Ome
 
     // ---- phase A: gather the K-vector of (Omega + L) + X, prox in place --------------------
     if (upper) {
-        const size_t e = (size_t)i * p + j;
+        const size_t e = gg_batch_offset(K, p) + (size_t)i * p + j;
 #pragma unroll 8
         for (int k = 0; k < K; ++k) {
             double v = Omega[k * pp + e];
@@ -289,12 +302,13 @@ prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Ome
     // iteration (the kernel is latency bound on these re-reads: ncu long-scoreboard 46 %).
     double acc[GG_NPART] = {0.0, 0.0, 0.0, 0.0, 0.0};
     {
+        const size_t qo = gg_batch_offset(K, p);
         const int sl0 = (I < J || tr <= tc) ? slot : (tc * PLD + tr);
         const bool ok0 = valid;
-        const size_t e0 = (size_t)i * p + j;
+        const size_t e0 = qo + (size_t)i * p + j;
         const int i1 = J * PT + tr, j1 = I * PT + tc;          // element of the mirror tile (J,I)
         const bool ok1 = (I < J) && (i1 < p) && (j1 < p);
-        const size_t e1 = (size_t)i1 * p + j1;
+        const size_t e1 = qo + (size_t)i1 * p + j1;
         const int sl1 = tc * PLD + tr;                         // = value of its transpose (j1, i1)
         if (ok0 || ok1) {
             const size_t ea = ok0 ? e0 : e1, eb = ok1 ? e1 : e0;   // keep addresses valid when one side is off
@@ -336,7 +350,7 @@ prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Ome
     if (!LATENT) {
         gg_block_sum<GG_NPART>(acc, scratch);
         if (threadIdx.x == 0) {
-            double* out = partials + ((size_t)I * nt + J) * GG_NPART;
+            double* out = partials + (((size_t)blockIdx.y * nt + I) * nt + J) * GG_NPART;
 #pragma unroll
             for (int q = 0; q < GG_NPART; ++q) out[q] = acc[q];
         }
@@ -350,7 +364,9 @@ __global__ void __launch_bounds__(EW_THREADS)
 build_w_upper_kernel(const double* __restrict__ Theta, double* __restrict__ X, const double* __restrict__ S,
                      const double* __restrict__ nk, const double* __restrict__ ctrl, int p, double* __restrict__ W)
 {
-    const int m = blockIdx.y;
+    // matrix k = blockIdx.y of problem q = blockIdx.z (K = gridDim.y matrices per problem)
+    const int m = blockIdx.z * gridDim.y + blockIdx.y;
+    ctrl += (size_t)blockIdx.z * GG_CTRL_STRIDE;
     if (ctrl[GG_C_DONE] != 0.0) return;
     const double rho = ctrl[GG_C_RHO];
     const double xs = ctrl[GG_C_XSCALE];
@@ -408,25 +424,31 @@ prox_mgl_upper_kernel(const double* __restrict__ Omega, const double* __restrict
 {
     extern __shared__ double ysm[];                 // K * UT_THREADS
     __shared__ double scratch[GG_NPART * 32];
-    if (ctrl[GG_C_DONE] != 0.0) return;
+    // problem q = blockIdx.y of a batch: control block q, matrices q*K.. (offset folded into the element index) and
+    // gridDim.x partial sums
+    const double* cq = ctrl + (size_t)blockIdx.y * GG_CTRL_STRIDE;
+    if (cq[GG_C_DONE] != 0.0) return;
     // tile rows are grouped by UT_C / UT_R = 4: the rows of group g start at tile column g
     const int nc = (p + UT_C - 1) / UT_C;
     constexpr int GR = UT_C / UT_R;
     int rem = blockIdx.x, g = 0;
     while (rem >= GR * (nc - g)) { rem -= GR * (nc - g); ++g; }
     const int I = g * GR + rem / (nc - g), J = g + rem % (nc - g);
-    const double inv_rho = 1.0 / ctrl[GG_C_RHO];
-    if (ctrl[GG_C_LAM1] > 0.0) { lambda1 = ctrl[GG_C_LAM1]; lambda2 = ctrl[GG_C_LAM2]; }
+    const double inv_rho = 1.0 / cq[GG_C_RHO];
+    if (cq[GG_C_LAM1] > 0.0) { lambda1 = cq[GG_C_LAM1]; lambda2 = cq[GG_C_LAM2]; }
     const double l1 = inv_rho * lambda1, l2 = inv_rho * lambda2;
     const int i = I * UT_R + threadIdx.x / UT_C, j = J * UT_C + threadIdx.x % UT_C;
     const size_t pp = (size_t)p * p;
     const bool own = (i < p) && (j < p) && (i <= j);
     double acc[GG_NPART] = {0.0, 0.0, 0.0, 0.0, 0.0};
     if (own) {
-        const size_t e = (size_t)i * p + j;
         double* y = ysm + threadIdx.x;
+        {
+            const size_t e = (size_t)i * p + j;
+            const size_t qo = gg_batch_offset(K, p);
 #pragma unroll 8
-        for (int k = 0; k < K; ++k) y[k * UT_THREADS] = Omega[k * pp + e] + X[k * pp + e];
+            for (int k = 0; k < K; ++k) y[k * UT_THREADS] = Omega[qo + k * pp + e] + X[qo + k * pp + e];
+        }
         if (i != j) {
             if (REG == 0) {            // GGL: group soft threshold of the l1-soft-thresholded vector
                 double ss = 0.0;
@@ -445,9 +467,10 @@ prox_mgl_upper_kernel(const double* __restrict__ Omega, const double* __restrict
             }
         }
         const double w = (i == j) ? 1.0 : 2.0;      // an off-diagonal entry stands for itself and its mirror image
+        const size_t e = (size_t)i * p + j;
 #pragma unroll 4
         for (int k = 0; k < K; ++k) {
-            const size_t o = (size_t)k * pp + e;
+            const size_t o = gg_batch_offset(K, p) + (size_t)k * pp + e;
             const double om = Omega[o], x = X[o], pv = Omega_prev[o];
             const double th = y[k * UT_THREADS];
             Theta[o] = th;
@@ -461,7 +484,7 @@ prox_mgl_upper_kernel(const double* __restrict__ Omega, const double* __restrict
     }
     gg_block_sum<GG_NPART>(acc, scratch);
     if (threadIdx.x == 0) {
-        double* out = partials + (size_t)blockIdx.x * GG_NPART;
+        double* out = partials + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * GG_NPART;
 #pragma unroll
         for (int q = 0; q < GG_NPART; ++q) out[q] = acc[q];
     }
@@ -991,7 +1014,7 @@ extern "C" int gg_mgl_ntile(int p) { return (p + PT - 1) / PT; }
 template <int REG, bool LATENT>
 static int launch_prox_mgl_t(const double* Omega, const double* Omega_prev, const double* L, double* X,
                              double* Theta, double* C, const double* ctrl, double l1, double l2, int K, int p,
-                             double* partials, cudaStream_t st)
+                             int nprob, double* partials, cudaStream_t st)
 {
     const int nt = gg_mgl_ntile(p);
     const size_t smem = (size_t)K * PSLOT * sizeof(double);
@@ -1002,7 +1025,7 @@ static int launch_prox_mgl_t(const double* Omega, const double* Omega_prev, cons
         if (e != cudaSuccess) return (int)e;
     }
     const int nst = (nt + 3) / 4;
-    dim3 grid(16 * (nst * (nst + 1) / 2));
+    dim3 grid(16 * (nst * (nst + 1) / 2), nprob);
     gg_count_launch(1);
     kern<<<grid, PT * PT, smem, st>>>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, partials);
     GG_CHECK_LAUNCH();
@@ -1010,23 +1033,23 @@ static int launch_prox_mgl_t(const double* Omega, const double* Omega_prev, cons
 }
 
 int gg_launch_prox_mgl(const double* Omega, const double* Omega_prev, const double* L, double* X, double* Theta,
-                       double* C, const double* ctrl, double l1, double l2, int reg, int K, int p,
+                       double* C, const double* ctrl, double l1, double l2, int reg, int K, int p, int nprob,
                        double* partials, cudaStream_t st)
 {
     const bool latent = (C != nullptr);
     if (reg == 0) {
-        return latent ? launch_prox_mgl_t<0, true>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, partials, st)
-                      : launch_prox_mgl_t<0, false>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, partials, st);
+        return latent ? launch_prox_mgl_t<0, true>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, nprob, partials, st)
+                      : launch_prox_mgl_t<0, false>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, nprob, partials, st);
     }
-    return latent ? launch_prox_mgl_t<1, true>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, partials, st)
-                  : launch_prox_mgl_t<1, false>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, partials, st);
+    return latent ? launch_prox_mgl_t<1, true>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, nprob, partials, st)
+                  : launch_prox_mgl_t<1, false>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, nprob, partials, st);
 }
 
 extern "C" int gg_mgl_upper_nparts(int p) { return ut_ntiles(p); }
 
 int gg_launch_prox_mgl_upper(const double* Omega, const double* Omega_prev, double* X, double* Theta,
-                             const double* ctrl, double l1, double l2, int reg, int K, int p, double* partials,
-                             cudaStream_t st)
+                             const double* ctrl, double l1, double l2, int reg, int K, int p, int nprob,
+                             double* partials, cudaStream_t st)
 {
     const size_t smem = (size_t)K * UT_THREADS * sizeof(double);
     if (smem > 200 * 1024) return -2;   // K too large for the shared-memory layout
@@ -1036,15 +1059,16 @@ int gg_launch_prox_mgl_upper(const double* Omega, const double* Omega_prev, doub
         if (e != cudaSuccess) return (int)e;
     }
     gg_count_launch(1);
-    kern<<<ut_ntiles(p), UT_THREADS, smem, st>>>(Omega, Omega_prev, X, Theta, ctrl, l1, l2, K, p, partials);
+    kern<<<dim3(ut_ntiles(p), nprob), UT_THREADS, smem, st>>>(Omega, Omega_prev, X, Theta, ctrl, l1, l2, K, p,
+                                                              partials);
     GG_CHECK_LAUNCH();
     return 0;
 }
 
 int gg_launch_build_w_upper(const double* Theta, double* X, const double* S, const double* nk, const double* ctrl,
-                            int K, int p, double* W, cudaStream_t st)
+                            int K, int p, int nprob, double* W, cudaStream_t st)
 {
-    dim3 grid((p + 1) / 2, K);
+    dim3 grid((p + 1) / 2, K, nprob);
     gg_count_launch(1);
     build_w_upper_kernel<<<grid, EW_THREADS, 0, st>>>(Theta, X, S, nk, ctrl, p, W);
     GG_CHECK_LAUNCH();

@@ -125,6 +125,21 @@ int gg_build_w_upper(const double* Theta, double* X, const double* S, const doub
                      int p, double* W, void* stream);
 int gg_mirror_upper(double* A0, double* A1, int M, int p, void* stream);
 
+/* Batches of nprob independent MGL problems of K instances each (ADMM_MGL_batch): the arrays are (nprob*K, p, p)
+ * stacks, problem q owns matrices q*K .. q*K+K-1, control block q (done flag, rho, pending X scale and lambda1 /
+ * lambda2 from ctrl[9..10], which must be set) and the partial sums at q * nparts * GG_NPART doubles, with nparts =
+ * gg_mgl_ntile(p)^2 (gg_prox_mgl_batch) or gg_mgl_upper_nparts(p) (gg_prox_mgl_upper_batch) -- the layout
+ * gg_stop_update reads for nprob problems.  Problems whose done flag is set are not touched.  Same kernels and
+ * arithmetic as the single-problem entry points, which are the case nprob = 1; nprob <= 65535. */
+int gg_prox_mgl_batch(const double* Omega, const double* Omega_prev, const double* L, double* X, double* Theta,
+                      double* C, const double* ctrl, double lambda1, double lambda2, int reg, int K, int p, int nprob,
+                      double* partials, void* stream);
+int gg_prox_mgl_upper_batch(const double* Omega, const double* Omega_prev, double* X, double* Theta, const double* ctrl,
+                            double lambda1, double lambda2, int reg, int K, int p, int nprob, double* partials,
+                            void* stream);
+int gg_build_w_upper_batch(const double* Theta, double* X, const double* S, const double* nk, const double* ctrl, int K,
+                           int p, int nprob, double* W, void* stream);
+
 /* K-sharded MGL (one process per GPU, SURVEY.md section 8e): V = (Omega + L) + X on the local instances
  * (L may be NULL), and the cross-instance prox on a row band: V, Theta are (K, nb, p) slabs holding global rows
  * row0..row0+nb-1 of all K instances (after the all-to-all re-tile).  Same prox as gg_prox_mgl. */
