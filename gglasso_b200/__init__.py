@@ -6,13 +6,15 @@ Drop-in replacements for ``gglasso.solver.admm_solver.ADMM_MGL``,
 ``install()`` rebinds those names inside an importable ``gglasso`` package so that
 ``glasso_problem`` and ``grid_search`` run unmodified on top of the GPU path.
 ``ADMM_MGL_batch`` (no counterpart in the reference, so ``install()`` leaves it alone) solves many MGL problems of the
-same shape in one device loop.
+same shape in one device loop.  ``stability_selection`` (also without counterpart) chooses lambda1 of SGL or MGL by
+StARS from raw samples, on the device.
 """
 from .solver.admm_solver import ADMM_MGL, ADMM_MGL_batch  # noqa: F401
 from .solver.single_admm_solver import ADMM_SGL, block_SGL, get_connected_components  # noqa: F401
 from .solver.functional_sgl_admm import ADMM_FSGL  # noqa: F401
 from .solver.ext_admm_solver import ext_ADMM_MGL  # noqa: F401
 from .solver.ppdna_solver import PPDNA, warmPPDNA  # noqa: F401
+from .stability import stability_selection  # noqa: F401
 from ._lib import GGLassoB200Error, LIB_PATH  # noqa: F401
 
 __version__ = "0.1.0"

@@ -69,6 +69,9 @@ SIGNATURES = {
     "gg_ppdna_cg_init": (_i, [_vp, _i, _i, _d, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gg_ppdna_cg": (_i, [_i, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                          _vp]),
+    "gg_subsample_cov": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "gg_edge_count": (_i, [_vp, _i, _i, _i, _i, _vp, _vp]),
+    "gg_stars_instability": (_i, [_vp, _i, _i, _i, _i, _vp, _vp]),
 }
 
 _LIB = None

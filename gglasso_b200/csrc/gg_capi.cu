@@ -66,6 +66,10 @@ int gg_launch_ppdna_cg_init(const double*, int, int, double, int, double*, doubl
 int gg_launch_ppdna_cg(int, const double*, const double*, const double*, const double*, const unsigned char*,
                        const double*, double, double, int, int, int, double*, double*, double*, double*, double*,
                        double*, double*, double*, cudaStream_t);
+int gg_launch_subsample_cov(const double*, const int*, const int*, const int*, int, int, int, int, double*, double*, int*,
+                            cudaStream_t);
+int gg_launch_edge_count(const double*, int, int, int, int, int*, cudaStream_t);
+int gg_launch_stars_instability(const int*, int, int, int, int, double*, cudaStream_t);
 
 #include <atomic>
 static std::atomic<long long> g_launches{0};
@@ -354,6 +358,27 @@ int gg_ppdna_cg(int iters, const double* Vt, const double* Q, const double* phi,
     if (iters < 0 || K <= 0 || p <= 0 || reg < 0 || reg > 1 || !(sigma > 0.0)) return -1;
     return gg_launch_ppdna_cg(iters, Vt, Q, phi, V, code, jscale, sigma, lambda1, reg, K, p, d, r, pv, q, Y, Z, cg,
                               partials, (cudaStream_t)stream);
+}
+
+int gg_subsample_cov(const double* X, const int* rowoff, const int* idx, const int* boff, int nsub, int K, int p,
+                     int scale, double* mean, double* S, int* zero_col, void* stream)
+{
+    if (nsub <= 0 || K <= 0 || p <= 0 || (long long)nsub * K > 65535 || !X || !rowoff || !idx || !boff || !mean || !S
+        || !zero_col)
+        return -1;
+    return gg_launch_subsample_cov(X, rowoff, idx, boff, nsub, K, p, scale, mean, S, zero_col, (cudaStream_t)stream);
+}
+
+int gg_edge_count(const double* Theta, int nsub, int L, int K, int p, int* counts, void* stream)
+{
+    if (nsub <= 0 || L <= 0 || K <= 0 || p <= 0 || (long long)L * K > 65535 || !Theta || !counts) return -1;
+    return gg_launch_edge_count(Theta, nsub, L, K, p, counts, (cudaStream_t)stream);
+}
+
+int gg_stars_instability(const int* counts, int L, int K, int p, int B, double* out, void* stream)
+{
+    if (L <= 0 || K <= 0 || p < 2 || B <= 0 || (long long)L * K > 2147483647LL || !counts || !out) return -1;
+    return gg_launch_stars_instability(counts, L, K, p, B, out, (cudaStream_t)stream);
 }
 
 }  // extern "C"

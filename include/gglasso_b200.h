@@ -253,6 +253,25 @@ int gg_ppdna_cg(int iters, const double* Vt, const double* Q, const double* phi,
                 double* d, double* r, double* pv, double* q, double* Y, double* Z, double* cg, double* partials,
                 void* stream);
 
+/* Stability selection (StARS, Liu, Roeder & Wasserman 2010; no reference counterpart).  The samples of K classes are
+ * one (sum n_k, p) FP64 array X, class k starting at row rowoff[k] (device int[K]).  A chunk of nsub subsamples is
+ * given by idx (device int): subsample s draws the b_k = boff[k+1] - boff[k] rows idx[s*boff[K] + boff[k] ..] (indices
+ * within class k) from class k; boff: device int[K+1], boff[0] = 0.
+ *  gg_subsample_cov    : S[s*K+k] = (1/b_k) Xc^T Xc with Xc the drawn rows of class k centred on their mean
+ *                        (np.cov(X_sub, rowvar=False, bias=True)), on FP64 tensor cores, exactly symmetric; scale != 0
+ *                        then divides by sqrt(S_ii) sqrt(S_jj) (the reference's scale_array_by_diagonal,
+ *                        src/gglasso/helper/basic_linalg.py).  S: (nsub*K, p, p); mean: nsub*K*p doubles of scratch;
+ *                        zero_col[s*K+k] (int, nsub*K) = smallest column whose drawn values are all equal (zero
+ *                        variance), or a value >= p if there is none.  nsub*K <= 65535.
+ *  gg_edge_count       : counts[l,k,i,j] += #{s < nsub : Theta[(s*L+l)*K+k][i][j] != 0} for i < j; counts (L,K,p,p)
+ *                        int32, zeroed by the caller once, entries i >= j untouched; deterministic (no atomics).
+ *  gg_stars_instability: per (l,k) of counts after B subsamples, theta = count/B: out[(l*K+k)*2] = sum_{i<j}
+ *                        2 theta (1 - theta) / C(p,2), out[(l*K+k)*2+1] = sum_{i<j} count / B; deterministic. */
+int gg_subsample_cov(const double* X, const int* rowoff, const int* idx, const int* boff, int nsub, int K, int p,
+                     int scale, double* mean, double* S, int* zero_col, void* stream);
+int gg_edge_count(const double* Theta, int nsub, int L, int K, int p, int* counts, void* stream);
+int gg_stars_instability(const int* counts, int L, int K, int p, int B, double* out, void* stream);
+
 /* Host-side execution of the exact device TV-prox routine (unit tests without a GPU). */
 void gg_host_tv1d(double* v, int n, int stride, double lam);
 
