@@ -132,11 +132,16 @@ gersh_rows_kernel(const double* __restrict__ A, int p, double* __restrict__ rowl
     if (i >= p) return;
     const double* a = A + (size_t)m * p * p + (size_t)i * p;
     double rs = 0.0;
-    for (int j = lane; j < p; j += 32) rs += fabs(a[j]);
+    for (int j = lane; j < p; j += 32)
+        if (j != i) rs += fabs(a[j]);
     rs = gg_warp_sum(rs);
     if (lane == 0) {
+        // The rounded sum can fall short of the exact off-diagonal sum by a relative (p-2)u, whatever the order;
+        // widened by 2pu (u = 2^-53) it no longer can, so rowlo is a true lower bound of the row's disc and a
+        // positive rowlo certifies positive definiteness.  (Summing |a_ii| into the row sum and subtracting it again
+        // would let that sum's rounding turn an exact bound <= 0 into a positive one.)
+        rs *= 1.0 + 2.0 * p * 1.1102230246251565e-16;
         const double d = a[i];
-        rs -= fabs(d);
         rowlo[(size_t)m * p + i] = d - rs;
         rowhi[(size_t)m * p + i] = d + rs;
     }
@@ -461,7 +466,8 @@ static int launch_round(double* G, int M, int p, int nb, int round, double tol, 
 }
 
 // A: (M,p,p) symmetric, overwritten by Vt (rows = eigenvectors, unit norm if `vectors`).
-// D: (M,p) eigenvalues (unsorted).  info[0] = sweeps used (block path) / max sweeps (small path).
+// D: (M,p) eigenvalues (unsorted).  info[0] = sweeps used (block path), 0 (small path: the per-matrix sweep counts
+// stay on the device, in the last slot of the workspace), -1 (tridiagonal path).
 int gg_eigh_impl(double* A, double* D, int M, int p, const double* ctrl, int mpp, void* ws, size_t ws_bytes,
                  int vectors, int block_nb2, double tol, int max_sweeps, double quad_tol, int* info,
                  double* Vwarm, cudaStream_t s)

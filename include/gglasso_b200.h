@@ -54,7 +54,8 @@ int gg_build_w(const double* Theta, const double* L, double* X, const double* S,
  * tridiagonalisation + divide & conquer + back-transformation.  block_nb2 = 0: default; 1: force the shared-memory
  * Jacobi kernel (p <= 160); 32/64/128: block-Jacobi with that many rows per block pair (p > 160).
  * tol<=0, max_sweeps<=0: defaults.  quad_tol: a sweep whose largest measured off-diagonal cosine is
- * below quad_tol is taken as the last one (quadratic convergence); 0 disables.  info[0] (host) = sweeps.
+ * below quad_tol is taken as the last one (quadratic convergence); 0 disables.  info[0] (host) = sweeps of the block
+ * Jacobi, 0 for the shared-memory Jacobi (its sweep counts are not copied back), -1 for the tridiagonal path.
  * Vt_warm (optional, (M,p,p), rows orthonormal; used for p <= 160): warm start from the eigenvectors of the
  * previous ADMM iteration (identity for the first call); overwritten with the new eigenvectors. */
 size_t gg_eigh_workspace_bytes(int M, int p);
