@@ -7,9 +7,10 @@ Drop-in replacements for ``gglasso.solver.admm_solver.ADMM_MGL``,
 ``glasso_problem`` and ``grid_search`` run unmodified on top of the GPU path.
 ``ADMM_MGL_batch`` (no counterpart in the reference, so ``install()`` leaves it alone) solves many MGL problems of the
 same shape in one device loop.  ``stability_selection`` (also without counterpart) chooses lambda1 of SGL or MGL by
-StARS from raw samples, on the device.
+StARS from raw samples, on the device.  ``block_MGL`` (also without counterpart) solves GGL / FGL component by
+component of an exact screening graph computed on the device, small components in ragged device batches.
 """
-from .solver.admm_solver import ADMM_MGL, ADMM_MGL_batch  # noqa: F401
+from .solver.admm_solver import ADMM_MGL, ADMM_MGL_batch, block_MGL, mgl_connected_components  # noqa: F401
 from .solver.single_admm_solver import ADMM_SGL, block_SGL, get_connected_components  # noqa: F401
 from .solver.functional_sgl_admm import ADMM_FSGL  # noqa: F401
 from .solver.ext_admm_solver import ext_ADMM_MGL  # noqa: F401

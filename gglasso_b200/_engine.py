@@ -271,10 +271,10 @@ class AdmmState:
         self.pvec = None
         if pvec is None:
             self.pdim = to_dev(np.full(self.nprob, mpp * ((p ** 2 + p) / 2)), dev)
-        else:                               # ragged batch of independent SGL problems padded to p
+        else:                               # ragged batch of independent problems, problem q padded from p_q to p
             pv = np.asarray(pvec, dtype=np.int64)
             self.pvec = torch.from_numpy(pv.astype(np.int32)).to(dev)
-            self.pdim = to_dev((pv ** 2 + pv) / 2.0, dev)
+            self.pdim = to_dev(mpp * ((pv ** 2 + pv) / 2.0), dev)
         self.stream = torch.cuda.current_stream().cuda_stream
 
     def reset(self, Omega_0, Theta_0=None, X_0=None, rho=1.0, lambdas=None):
@@ -442,6 +442,10 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
     problem q owning matrices q*K .. q*K+K-1 and control block q; ``lambda1`` / ``lambda2`` may be arrays of one value
     per problem.  Default: one problem of all M matrices.
 
+    ``pvec``: one true size p_q <= p per problem of a ragged batch whose problems are padded to p with decoupled unit
+    diagonal entries (S = Omega = Theta = I, X = 0); the padding is left out of the residual norms.  'sgl' (block_SGL)
+    or non-latent 'mgl' with the Boyd criterion (block_MGL, always on full matrices).
+
     ``state``: an AdmmState of the same shapes from an earlier call (lambda grids): its buffers, workspace and captured
     iteration graphs are reused.  ``graph``: run the iterations as replays of two captured CUDA graphs (one per
     Omega ping-pong direction).  Off by default (GG_GRAPH=1 turns it on for p <= GG_GRAPH_MAX_P): measured on B200 the
@@ -457,6 +461,9 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
             raise NotImplementedError("a batch of MGL problems supports stopping_criterion='boyd' without measure only")
         if mpp > K_TILE_MAX:
             raise NotImplementedError(f"a batch of MGL problems needs K <= {K_TILE_MAX} (tile-pair prox), got K = {mpp}")
+    if kind == "mgl" and pvec is not None and (latent or measure or stopping_criterion != "boyd" or mpp > K_TILE_MAX):
+        raise NotImplementedError(f"a ragged batch of MGL problems supports the non-latent loop with "
+                                  f"stopping_criterion='boyd' without measure and K <= {K_TILE_MAX} only")
     if state is not None:
         st = state
         assert st.M == M and st.p == p and st.mpp == mpp and st.latent == latent and st.hist_cap >= max_iter
@@ -490,6 +497,11 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
     else:
         nparts_fused = lib.gg_sgl_nparts(p, M)
     prox_mgl_fn = lib.gg_prox_mgl_batch
+    ragged_mgl = kind == "mgl" and st.pvec is not None
+    if ragged_mgl:
+        def prox_mgl_fn(Omega, Omega_prev, L, X, Theta, C, *args):      # non-latent: L and C are None
+            *args, parts, sm = args
+            return lib.gg_prox_mgl_ragged(Omega, Omega_prev, X, Theta, *args, _p(st.pvec), parts, sm)
     nparts_dual = lib.gg_sgl_nparts(p, M) * mpp
     # K beyond the shared-memory layout of the fused tile-pair prox (K x 272 doubles per CTA): the row-band prox of the
     # K-sharded path takes over on one device (pack -> band prox -> unpack fused with the dual update)
@@ -500,8 +512,9 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
     # Non-latent MGL on the tridiagonal eigensolver path: the iterations keep only the UPPER triangles of Theta, X and W
     # current (every consumer inside the loop reads nothing else; half the elementwise HBM traffic) and the lower
     # triangles are filled once after the loop -- prox_p's mirroring (ggl_helper.py:198-205) done once.
-    upper = (kind == "mgl" and not latent and not big_K and stopping_criterion == "boyd" and not measure
-             and not _DEBUG_KEEP_INPUT and st.eig.nb2 == 0 and p > lib.gg_jacobi_max()
+    # A ragged batch stays on full matrices (its components are <= 160, where the upper-triangle path saves little).
+    upper = (kind == "mgl" and not latent and not big_K and not ragged_mgl and stopping_criterion == "boyd"
+             and not measure and not _DEBUG_KEEP_INPUT and st.eig.nb2 == 0 and p > lib.gg_jacobi_max()
              and _env_int("GG_UPPER", 1) != 0)
     nparts_upper = lib.gg_mgl_upper_nparts(p) if kind == "mgl" else 0
     if upper:

@@ -41,6 +41,8 @@ SIGNATURES = {
     "gg_prox_mgl": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _vp, _vp]),
     "gg_prox_mgl_batch": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _i, _vp, _vp]),
     "gg_prox_mgl_upper_batch": (_i, [_vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _i, _vp, _vp]),
+    "gg_prox_mgl_ragged": (_i, [_vp, _vp, _vp, _vp, _vp, _d, _d, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "gg_mgl_screen": (_i, [_vp, _vp, _d, _d, _i, _i, _i, _vp, _vp]),
     "gg_build_w_upper_batch": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
     "gg_add3": (_i, [_vp, _vp, _vp, _vp, _sz, _vp]),
     "gg_pack_bands": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp]),

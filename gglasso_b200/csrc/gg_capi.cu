@@ -11,6 +11,9 @@ int gg_launch_dual_update(double*, const double*, const double*, const double*, 
                           int, int, int, double*, cudaStream_t);
 int gg_launch_prox_mgl(const double*, const double*, const double*, double*, double*, double*, const double*, double,
                        double, int, int, int, int, double*, cudaStream_t);
+int gg_launch_prox_mgl_ragged(const double*, const double*, double*, double*, const double*, double, double, int, int,
+                              int, int, const int*, double*, cudaStream_t);
+int gg_launch_mgl_screen(const double*, const double*, double, double, int, int, int, uint32_t*, cudaStream_t);
 int gg_launch_prox_mgl_upper(const double*, const double*, double*, double*, const double*, double, double, int, int,
                              int, int, double*, cudaStream_t);
 int gg_launch_build_w_upper(const double*, double*, const double*, const double*, const double*, int, int, int,
@@ -153,6 +156,24 @@ int gg_prox_mgl_batch(const double* Omega, const double* Omega_prev, const doubl
     if (K <= 0 || p <= 0 || nprob <= 0 || nprob > 65535 || reg < 0 || reg > 1 || ctrl == nullptr) return -1;
     return gg_launch_prox_mgl(Omega, Omega_prev, L, X, Theta, C, ctrl, lambda1, lambda2, reg, K, p, nprob, partials,
                               (cudaStream_t)stream);
+}
+
+int gg_prox_mgl_ragged(const double* Omega, const double* Omega_prev, double* X, double* Theta, const double* ctrl,
+                       double lambda1, double lambda2, int reg, int K, int p, int nprob, const int* pvec,
+                       double* partials, void* stream)
+{
+    if (K <= 0 || p <= 0 || nprob <= 0 || nprob > 65535 || reg < 0 || reg > 1 || ctrl == nullptr || pvec == nullptr
+        || partials == nullptr)
+        return -1;
+    return gg_launch_prox_mgl_ragged(Omega, Omega_prev, X, Theta, ctrl, lambda1, lambda2, reg, K, p, nprob, pvec,
+                                     partials, (cudaStream_t)stream);
+}
+
+int gg_mgl_screen(const double* S, const double* nk, double lambda1, double lambda2, int reg, int K, int p,
+                  uint32_t* adj, void* stream)
+{
+    if (K <= 0 || p <= 0 || reg < 0 || reg > 1 || S == nullptr || adj == nullptr) return -1;
+    return gg_launch_mgl_screen(S, nk, lambda1, lambda2, reg, K, p, adj, (cudaStream_t)stream);
 }
 
 int gg_prox_mgl_upper(const double* Omega, const double* Omega_prev, double* X, double* Theta, const double* ctrl,

@@ -6,6 +6,7 @@
 //   gg_prox_mgl       Theta = prox_p(Omega+L+X, l1/rho, l2/rho)   admm_solver.py:190-194, ggl_helper.py:190-207
 //                     GGL: ggl_helper.py:68-71,38-43; FGL: ggl_helper.py:131-134 + fgl_helper.py:11-68
 //                     same fusion; one CTA per 16x16 tile pair (I<=J), all K instances, mirrored write
+//   gg_prox_mgl_ragged  the same for a ragged batch (block_MGL): padding left out of the partial sums
 //   gg_dual_update    X += Omega - Theta + L + partial sums (latent) admm_solver.py:208, single_admm_solver.py:177
 //   gg_stop_update    Boyd residuals, stopping test, rho update    admm_solver.py:216-246,316-331
 //   gg_scale          X *= pending rho_old/rho_new                 admm_solver.py:236
@@ -232,12 +233,15 @@ __device__ __forceinline__ size_t gg_batch_offset(int K, int p)
     return (size_t)q * K * ((size_t)p * p);
 }
 
-template <int REG, bool LATENT>
-__global__ void __launch_bounds__(PT * PT)
-prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Omega_prev,
-                const double* __restrict__ L, double* __restrict__ X, double* __restrict__ Theta,
-                double* __restrict__ C, const double* __restrict__ ctrl, double lambda1, double lambda2,
-                int K, int p, double* __restrict__ partials)
+// Body of the tile-pair prox kernels.  RAGGED: problem q of the batch is a p_q x p_q problem (p_q = pvec[q]) padded to
+// p with decoupled unit diagonal entries; the padding is prox'd like any entry (it stays a fixed point) but is left out
+// of the five partial sums, as prox_sgl_kernel does with its pvec.
+template <int REG, bool LATENT, bool RAGGED>
+__device__ __forceinline__ void
+prox_mgl_body(const double* __restrict__ Omega, const double* __restrict__ Omega_prev,
+              const double* __restrict__ L, double* __restrict__ X, double* __restrict__ Theta,
+              double* __restrict__ C, const double* __restrict__ ctrl, double lambda1, double lambda2,
+              int K, int p, double* __restrict__ partials, const int* __restrict__ pvec)
 {
     extern __shared__ double ysm[];                 // K * PSLOT
     __shared__ double scratch[GG_NPART * 32];
@@ -310,6 +314,12 @@ prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Ome
         const bool ok1 = (I < J) && (i1 < p) && (j1 < p);
         const size_t e1 = qo + (size_t)i1 * p + j1;
         const int sl1 = tc * PLD + tr;                         // = value of its transpose (j1, i1)
+        bool in0 = true, in1 = true;                           // entries that count in the partial sums
+        if (RAGGED) {
+            const int pb = pvec[blockIdx.y];
+            in0 = (i < pb) && (j < pb);
+            in1 = (i1 < pb) && (j1 < pb);
+        }
         if (ok0 || ok1) {
             const size_t ea = ok0 ? e0 : e1, eb = ok1 ? e1 : e0;   // keep addresses valid when one side is off
 #pragma unroll (LATENT ? 4 : 2)
@@ -329,7 +339,9 @@ prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Ome
                         const double xn = x0 + d1;             // X += Omega - Theta (+ L = 0)
                         X[o + e0] = xn;
                         const double d2 = om0 - p0;
-                        acc[0] += om0 * om0; acc[1] += th0 * th0; acc[2] += xn * xn; acc[3] += d1 * d1; acc[4] += d2 * d2;
+                        if (!RAGGED || in0) {
+                            acc[0] += om0 * om0; acc[1] += th0 * th0; acc[2] += xn * xn; acc[3] += d1 * d1; acc[4] += d2 * d2;
+                        }
                     }
                 }
                 if (ok1) {
@@ -341,7 +353,9 @@ prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Ome
                         const double xn = x1 + d1;
                         X[o + e1] = xn;
                         const double d2 = om1 - p1;
-                        acc[0] += om1 * om1; acc[1] += th1 * th1; acc[2] += xn * xn; acc[3] += d1 * d1; acc[4] += d2 * d2;
+                        if (!RAGGED || in1) {
+                            acc[0] += om1 * om1; acc[1] += th1 * th1; acc[2] += xn * xn; acc[3] += d1 * d1; acc[4] += d2 * d2;
+                        }
                     }
                 }
             }
@@ -355,6 +369,29 @@ prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Ome
             for (int q = 0; q < GG_NPART; ++q) out[q] = acc[q];
         }
     }
+}
+
+template <int REG, bool LATENT>
+__global__ void __launch_bounds__(PT * PT)
+prox_mgl_kernel(const double* __restrict__ Omega, const double* __restrict__ Omega_prev,
+                const double* __restrict__ L, double* __restrict__ X, double* __restrict__ Theta,
+                double* __restrict__ C, const double* __restrict__ ctrl, double lambda1, double lambda2,
+                int K, int p, double* __restrict__ partials)
+{
+    prox_mgl_body<REG, LATENT, false>(Omega, Omega_prev, L, X, Theta, C, ctrl, lambda1, lambda2, K, p, partials,
+                                      nullptr);
+}
+
+// ragged batch of non-latent problems (block_MGL): pvec[q] = true size of problem q
+template <int REG>
+__global__ void __launch_bounds__(PT * PT)
+prox_mgl_ragged_kernel(const double* __restrict__ Omega, const double* __restrict__ Omega_prev,
+                       double* __restrict__ X, double* __restrict__ Theta, const double* __restrict__ ctrl,
+                       double lambda1, double lambda2, int K, int p, const int* __restrict__ pvec,
+                       double* __restrict__ partials)
+{
+    prox_mgl_body<REG, false, true>(Omega, Omega_prev, nullptr, X, Theta, nullptr, ctrl, lambda1, lambda2, K, p,
+                                    partials, pvec);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1043,6 +1080,26 @@ int gg_launch_prox_mgl(const double* Omega, const double* Omega_prev, const doub
     }
     return latent ? launch_prox_mgl_t<1, true>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, nprob, partials, st)
                   : launch_prox_mgl_t<1, false>(Omega, Omega_prev, L, X, Theta, C, ctrl, l1, l2, K, p, nprob, partials, st);
+}
+
+int gg_launch_prox_mgl_ragged(const double* Omega, const double* Omega_prev, double* X, double* Theta,
+                              const double* ctrl, double l1, double l2, int reg, int K, int p, int nprob,
+                              const int* pvec, double* partials, cudaStream_t st)
+{
+    const int nt = gg_mgl_ntile(p);
+    const size_t smem = (size_t)K * PSLOT * sizeof(double);
+    if (smem > 200 * 1024) return -2;   // K too large for the shared-memory layout
+    auto kern = reg == 0 ? prox_mgl_ragged_kernel<0> : prox_mgl_ragged_kernel<1>;
+    if (smem > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return (int)e;
+    }
+    const int nst = (nt + 3) / 4;
+    dim3 grid(16 * (nst * (nst + 1) / 2), nprob);
+    gg_count_launch(1);
+    kern<<<grid, PT * PT, smem, st>>>(Omega, Omega_prev, X, Theta, ctrl, l1, l2, K, p, pvec, partials);
+    GG_CHECK_LAUNCH();
+    return 0;
 }
 
 extern "C" int gg_mgl_upper_nparts(int p) { return ut_ntiles(p); }

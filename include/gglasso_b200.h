@@ -22,6 +22,7 @@
 #define GGLASSO_B200_H
 
 #include <stddef.h>
+#include <stdint.h>
 
 #ifdef __cplusplus
 extern "C" {
@@ -140,6 +141,20 @@ int gg_prox_mgl_upper_batch(const double* Omega, const double* Omega_prev, doubl
                             void* stream);
 int gg_build_w_upper_batch(const double* Theta, double* X, const double* S, const double* nk, const double* ctrl, int K,
                            int p, int nprob, double* W, void* stream);
+
+/* Ragged batch of non-latent MGL problems (block_MGL): gg_prox_mgl_batch's layout, arithmetic and Theta / X, with
+ * problem q a pvec[q] x pvec[q] problem padded to p (padding S = Omega = Theta = I, X = 0, a fixed point of the
+ * iteration): entries with i >= pvec[q] or j >= pvec[q] are left out of the five partial sums. */
+int gg_prox_mgl_ragged(const double* Omega, const double* Omega_prev, double* X, double* Theta, const double* ctrl,
+                       double lambda1, double lambda2, int reg, int K, int p, int nprob, const int* pvec,
+                       double* partials, void* stream);
+
+/* Exact component screen of MGL (reg 0 = GGL, 1 = FGL; K <= 90): adj (p rows of ceil(p/32) uint32 words) gets bit b
+ * of word w in row i set iff j = 32 w + b > i and prox_P(s_ij) != 0 with s_ij = (nk[k] S_k[i][j])_k (nk == NULL:
+ * weights 1) and P the prox penalty at rho = 1 (same routines and expressions as gg_prox_mgl).  Every other bit
+ * (diagonal, lower triangle, tail past p) is 0.  Deterministic. */
+int gg_mgl_screen(const double* S, const double* nk, double lambda1, double lambda2, int reg, int K, int p,
+                  uint32_t* adj, void* stream);
 
 /* K-sharded MGL (one process per GPU, SURVEY.md section 8e): V = (Omega + L) + X on the local instances
  * (L may be NULL), and the cross-instance prox on a row band: V, Theta are (K, nb, p) slabs holding global rows
