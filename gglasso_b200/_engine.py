@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import CTRL_STRIDE, HIST_STRIDE, NPART, C_DONE, C_ITER, C_RHO, C_STATUS, C_LAM1, C_LAM2
+from ._lib import CTRL_STRIDE, HIST_STRIDE, NPART, C_DONE, C_ITER, C_RHO, C_XSCALE, C_STATUS, C_LAM1, C_LAM2
 
 
 # largest K of the fused tile-pair MGL prox (K x 272 doubles of shared memory per CTA <= 200 KB)
@@ -27,6 +27,33 @@ K_TILE_MAX = 90
 
 def _p(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
+
+
+def control_block(nprob, rho, lambdas=None):
+    """fresh host control block of ``nprob`` problems (float64, (nprob, CTRL_STRIDE)): rho, no pending dual rescale and,
+    for MGL, ``lambdas`` = (lambda1, lambda2), each a scalar or one value per problem."""
+    ctrl = np.zeros((nprob, CTRL_STRIDE))
+    ctrl[:, C_RHO] = rho
+    ctrl[:, C_XSCALE] = 1.0
+    if lambdas is not None:
+        ctrl[:, C_LAM1], ctrl[:, C_LAM2] = lambdas
+    return ctrl
+
+
+def boyd_status(ctrl, hist):
+    """the reference's status of one problem after the 'boyd' loop, and its residual series max(r_t, s_t).
+    ``ctrl``: the problem's control block row; ``hist``: its residual history, one row per iteration."""
+    n = int(ctrl[C_ITER])
+    r, s, e_pri, e_dual = hist[n - 1, :4]
+    if ctrl[C_DONE] != 0:
+        status = "optimal"
+    elif r <= e_pri:
+        status = "primal optimal"
+    elif s <= e_dual:
+        status = "dual optimal"
+    else:
+        status = "max iterations reached"
+    return status, np.maximum(hist[:n, 0], hist[:n, 1])
 
 
 def _env_int(name, default):
@@ -231,10 +258,11 @@ def eigh(A, nb2=None):
 
 
 class AdmmState:
-    """Device buffers of one batched ADMM run: M matrices, ``mpp`` per problem."""
+    """Device buffers of one batched ADMM run: M matrices, ``mpp`` per problem.  ``lambdas`` (MGL): (lambda1, lambda2)
+    for the control block, where the MGL kernels read them (see control_block)."""
 
     def __init__(self, S, Omega_0, Theta_0, X_0, mpp, rho, max_iter, latent, nk=None, mu=None, lam_mat=None,
-                 pvec=None):
+                 pvec=None, lambdas=None):
         self.lib = _lib.load()
         self.dev = dev = require_cuda()
         self.S = to_dev(S, dev)
@@ -245,7 +273,6 @@ class AdmmState:
         self.Omega = to_dev(Omega_0, dev)
         self.Omega_new = torch.empty_like(self.Omega)
         self._bufA, self._bufB = self.Omega, self.Omega_new
-        self.nswap = 0
         # defaults of the reference (admm_solver.py:143-146) are formed on the device: no extra uploads
         self.Theta = self.Omega.clone() if Theta_0 is None else to_dev(Theta_0, dev)
         self.X = torch.zeros_like(self.S) if X_0 is None else to_dev(X_0, dev)
@@ -261,10 +288,7 @@ class AdmmState:
         self.nk = None if nk is None else to_dev(nk, dev)
         self.mu = None if mu is None else to_dev(mu, dev)
         self.lam_mat = None if lam_mat is None else to_dev(lam_mat, dev)
-        ctrl = np.zeros((self.nprob, CTRL_STRIDE))
-        ctrl[:, C_RHO] = rho
-        ctrl[:, 1] = 1.0
-        self.ctrl = to_dev(ctrl, dev)
+        self.ctrl = to_dev(control_block(self.nprob, rho, lambdas), dev)
         self.hist_cap = max_iter
         self.hist = torch.zeros((self.nprob, max_iter, HIST_STRIDE), dtype=torch.float64, device=dev)
         p = self.p
@@ -278,11 +302,10 @@ class AdmmState:
         self.stream = torch.cuda.current_stream().cuda_stream
 
     def reset(self, Omega_0, Theta_0=None, X_0=None, rho=1.0, lambdas=None):
-        """re-arm the state for another solve of the same shape on the same buffers (lambda grids): captured CUDA
-        graphs of the iteration stay valid.  ``lambdas`` = (lambda1, lambda2) go into the control block."""
+        """re-arm the state for another solve of the same shape on the same buffers (lambda grids).
+        ``lambdas`` = (lambda1, lambda2) go into the control block."""
         if self.Omega is not self._bufA:
             self.Omega, self.Omega_new = self._bufA, self._bufB
-        self.nswap = 0
         self.Omega.copy_(Omega_0 if isinstance(Omega_0, torch.Tensor) else to_dev(Omega_0, self.dev))
         if Theta_0 is None:
             self.Theta.copy_(self.Omega)
@@ -294,12 +317,7 @@ class AdmmState:
             self.X.copy_(X_0 if isinstance(X_0, torch.Tensor) else to_dev(X_0, self.dev))
         if self.L is not None:
             self.L.zero_()
-        ctrl = np.zeros((self.nprob, CTRL_STRIDE))
-        ctrl[:, C_RHO] = rho
-        ctrl[:, 1] = 1.0
-        if lambdas is not None:
-            ctrl[:, C_LAM1], ctrl[:, C_LAM2] = lambdas
-        self.ctrl.copy_(torch.from_numpy(ctrl), non_blocking=False)
+        self.ctrl.copy_(torch.from_numpy(control_block(self.nprob, rho, lambdas)), non_blocking=False)
         self.hist.zero_()
 
     # -- one Omega step: W build, eigh, phi+ reconstruction into Omega_new -----------------
@@ -327,7 +345,6 @@ class AdmmState:
 
     def swap(self):
         self.Omega, self.Omega_new = self.Omega_new, self.Omega
-        self.nswap += 1
 
     def final_omega(self, iters):
         """Omega of problem q lives in the buffer written by its last *executed* iteration (kernels are
@@ -360,14 +377,8 @@ class AdmmState:
               primal residual r -- available for the non-latent 'boyd' loop;
           (2) a positive Gershgorin lower bound;
         otherwise the exact smallest eigenvalue is computed (min_eig)."""
-        if res is not None and not self.latent and res.get("D_is_W") and self.nprob == 1:
-            n = int(res["iters"][0])
-            r, rho_used = res["hist"][0, n - 1, 0], res["hist"][0, n - 1, 4]
-            beta = (self.nk if self.nk is not None else torch.ones(self.M, dtype=torch.float64, device=self.dev)) / rho_used
-            dmin = self.eig.D.min(dim=1).values
-            lam_min_omega = 0.5 * (torch.sqrt(dmin * dmin + 4 * beta) + dmin)
-            if float(lam_min_omega.min().item()) - float(r) > 0.0:
-                return True, None
+        if self._weyl_certified(res):
+            return True, None
         out = torch.empty(self.M, dtype=torch.float64, device=self.dev)
         _lib.check(self.lib.gg_gershgorin_min(_p(A), self.M, self.p, _p(self.eig.ws), self.eig.ws_bytes, _p(out),
                                               self.stream), "gg_gershgorin_min")
@@ -380,17 +391,25 @@ class AdmmState:
         """like is_posdef, but when an eigendecomposition is needed it is only ENQUEUED (tridiagonal path: no host
         synchronisation) and a device scalar is returned, so the caller can overlap it with the D2H copies of the
         solution.  Returns None (certified PD) or a 0-d device tensor holding the smallest eigenvalue."""
-        if res is not None and not self.latent and res.get("D_is_W") and self.nprob == 1:
-            n = int(res["iters"][0])
-            r, rho_used = res["hist"][0, n - 1, 0], res["hist"][0, n - 1, 4]
-            beta = (self.nk if self.nk is not None else torch.ones(self.M, dtype=torch.float64, device=self.dev)) / rho_used
-            dmin = self.eig.D.min(dim=1).values
-            lam_min_omega = 0.5 * (torch.sqrt(dmin * dmin + 4 * beta) + dmin)
-            if float(lam_min_omega.min().item()) - float(r) > 0.0:
-                return None
-        B = A.clone()
-        D = self.eig.eigh(B, ctrl=None, mpp=1, vectors=0, stream=self.stream)
-        return D.min()
+        if self._weyl_certified(res):
+            return None
+        return self.eigvalsh(A).min()
+
+    def _weyl_certified(self, res):
+        """certificate (1) of is_posdef, from the loop's info ``res``: lambda_min(Omega) - r > 0"""
+        if res is None or self.latent or not res.get("D_is_W") or self.nprob != 1:
+            return False
+        n = int(res["iters"][0])
+        r, rho_used = res["hist"][0, n - 1, 0], res["hist"][0, n - 1, 4]
+        beta = (self.nk if self.nk is not None else torch.ones(self.M, dtype=torch.float64, device=self.dev)) / rho_used
+        dmin = self.eig.D.min(dim=1).values
+        lam_min_omega = 0.5 * (torch.sqrt(dmin * dmin + 4 * beta) + dmin)
+        return float(lam_min_omega.min().item()) - float(r) > 0.0
+
+    def eigvalsh(self, A):
+        """eigenvalues (M, p), unordered, of every matrix of the stack A; A is left intact (the eigensolver works on a
+        copy).  Only enqueued; the result is the workspace's D, overwritten by the next decomposition."""
+        return self.eig.eigh(A.clone(), ctrl=None, mpp=1, vectors=0, stream=self.stream)
 
     def min_eig_per_problem(self, A):
         """smallest eigenvalue of each problem's matrices in A, or -- where the Gershgorin bound of all of them is
@@ -402,7 +421,7 @@ class AdmmState:
         g = g.reshape(self.nprob, -1).amin(dim=1)
         if bool((g > 0.0).all().item()):
             return g
-        D = self.eig.eigh(A.clone(), ctrl=None, mpp=1, vectors=0, stream=self.stream)
+        D = self.eigvalsh(A)
         return torch.where(g > 0.0, g, D.reshape(self.nprob, -1).amin(dim=1))
 
     def mark(self):
@@ -427,15 +446,13 @@ class AdmmState:
 
     def min_eig(self, A):
         """smallest eigenvalue over the stack (post-loop PD checks; reference uses eigvalsh)."""
-        B = A.clone()
-        D = self.eig.eigh(B, ctrl=None, mpp=1, vectors=0, stream=self.stream)
-        return float(D.min().item())
+        return float(self.eigvalsh(A).min().item())
 
 
 def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None, lam_mat=None, rho=1.0,
              max_iter=1000, tol=1e-7, rtol=1e-4, stopping_criterion="boyd", update_rho=True, verbose=False,
              measure=False, latent=False, mu=None, nk=None, header=None, check_every=None, trace=None,
-             check_symmetric=False, pvec=None, Mblk=None, print_rho=False, state=None, graph=None, K=None):
+             check_symmetric=False, pvec=None, Mblk=None, print_rho=False, state=None, K=None):
     """Run the device ADMM loop.  ``kind``: 'mgl' (one problem of K matrices) or 'sgl' (M problems).
 
     ``K`` ('mgl' only): matrices per problem.  The stacks then hold M/K independent MGL problems (ADMM_MGL_batch),
@@ -446,11 +463,8 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
     diagonal entries (S = Omega = Theta = I, X = 0); the padding is left out of the residual norms.  'sgl' (block_SGL)
     or non-latent 'mgl' with the Boyd criterion (block_MGL, always on full matrices).
 
-    ``state``: an AdmmState of the same shapes from an earlier call (lambda grids): its buffers, workspace and captured
-    iteration graphs are reused.  ``graph``: run the iterations as replays of two captured CUDA graphs (one per
-    Omega ping-pong direction).  Off by default (GG_GRAPH=1 turns it on for p <= GG_GRAPH_MAX_P): measured on B200 the
-    loop is bound by the GPU-side latency of the eigensolver's dependent launches, not by the host -- cfg1 23.0 ms
-    eager vs 29.7 ms with capture + instantiation, cfg4 grid 2.65 s vs 2.60 s (profiles/r02_small_configs.json).
+    ``state``: an AdmmState of the same shapes from an earlier call (lambda grids): its buffers and eigensolver
+    workspace are reused.
     Returns (state, info) where info carries iteration counts, status and histories (numpy).
     """
     S3 = S if S.ndim == 3 else S[None]       # numpy arrays or device tensors
@@ -464,26 +478,17 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
     if kind == "mgl" and pvec is not None and (latent or measure or stopping_criterion != "boyd" or mpp > K_TILE_MAX):
         raise NotImplementedError(f"a ragged batch of MGL problems supports the non-latent loop with "
                                   f"stopping_criterion='boyd' without measure and K <= {K_TILE_MAX} only")
+    lambdas = (lambda1, lambda2) if kind == "mgl" else None      # the MGL kernels read them from the control block
     if state is not None:
         st = state
         assert st.M == M and st.p == p and st.mpp == mpp and st.latent == latent and st.hist_cap >= max_iter
         st.reset(Omega_0.reshape(S3.shape), None if Theta_0 is None else Theta_0.reshape(S3.shape),
-                 None if X_0 is None else X_0.reshape(S3.shape), rho,
-                 lambdas=(lambda1, lambda2) if kind == "mgl" else None)
+                 None if X_0 is None else X_0.reshape(S3.shape), rho, lambdas=lambdas)
         st.stream = torch.cuda.current_stream().cuda_stream
     else:
         st = AdmmState(S3, Omega_0.reshape(S3.shape), None if Theta_0 is None else Theta_0.reshape(S3.shape),
                        None if X_0 is None else X_0.reshape(S3.shape), mpp, rho, max_iter, latent, nk=nk, mu=mu,
-                       lam_mat=lam_mat, pvec=pvec)
-        if kind == "mgl":                        # lambdas live in the control block (see GG_C_LAM1)
-            if np.ndim(lambda1) == 0 and np.ndim(lambda2) == 0:
-                st.ctrl[:, C_LAM1] = lambda1
-                st.ctrl[:, C_LAM2] = lambda2
-            else:                                # one value per problem of a batch
-                lam = np.broadcast_to(np.stack(np.broadcast_arrays(np.asarray(lambda1, dtype=np.float64),
-                                                                   np.asarray(lambda2, dtype=np.float64)), -1),
-                                      (st.nprob, 2))
-                st.ctrl[:, C_LAM1:C_LAM2 + 1] = torch.from_numpy(np.array(lam)).to(st.dev)
+                       lam_mat=lam_mat, pvec=pvec, lambdas=lambdas)
     lib, stream = st.lib, st.stream
     nprob = st.nprob
     regi = {"GGL": 0, "FGL": 1}.get(reg, -1)
@@ -496,12 +501,7 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
         nparts_fused = nt * nt
     else:
         nparts_fused = lib.gg_sgl_nparts(p, M)
-    prox_mgl_fn = lib.gg_prox_mgl_batch
     ragged_mgl = kind == "mgl" and st.pvec is not None
-    if ragged_mgl:
-        def prox_mgl_fn(Omega, Omega_prev, L, X, Theta, C, *args):      # non-latent: L and C are None
-            *args, parts, sm = args
-            return lib.gg_prox_mgl_ragged(Omega, Omega_prev, X, Theta, *args, _p(st.pvec), parts, sm)
     nparts_dual = lib.gg_sgl_nparts(p, M) * mpp
     # K beyond the shared-memory layout of the fused tile-pair prox (K x 272 doubles per CTA): the row-band prox of the
     # K-sharded path takes over on one device (pack -> band prox -> unpack fused with the dual update)
@@ -520,18 +520,15 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
     if upper:
         nparts_fused = nparts_upper
     nparts = nparts_dual if (latent or big_K) else nparts_fused
-    if not hasattr(st, "_loopbuf"):          # loop buffers live with the state, so that captured graphs can be reused
-        vband = tband = blk_nrm = None
-        if big_K:
-            vband = torch.empty(M * p * p, dtype=torch.float64, device=st.dev)
-            tband = torch.zeros(M * p * p, dtype=torch.float64, device=st.dev)
-        partials = torch.zeros((nprob, max(nparts_fused, nparts_dual, nparts_upper), NPART), dtype=torch.float64,
-                               device=st.dev)
-        if Mblk is not None:
-            blk_nrm = torch.zeros((M, (p // Mblk) ** 2), dtype=torch.float64, device=st.dev)
-        st._loopbuf = (vband, tband, partials, blk_nrm)
-        st._graphs = {}
-    vband, tband, partials, blk_nrm = st._loopbuf
+    vband = tband = blk_nrm = None
+    if big_K:
+        vband = torch.empty(M * p * p, dtype=torch.float64, device=st.dev)
+        tband = torch.zeros(M * p * p, dtype=torch.float64, device=st.dev)
+    partials = torch.zeros((nprob, max(nparts_fused, nparts_dual, nparts_upper), NPART), dtype=torch.float64,
+                           device=st.dev)
+    if Mblk is not None:
+        blk_nrm = torch.zeros((M, (p // Mblk) ** 2), dtype=torch.float64, device=st.dev)
+    C = st.W if latent else None         # latent: the prox also forms C = Theta - X - Omega in W for the L step
     if check_every is None:
         check_every = 1 if (measure or verbose or p > 400) else 4
     runtime = np.zeros(max_iter)
@@ -551,96 +548,7 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
             print("%4s\t%10s" % ("iter", "kkt residual"))
     printed = 0
 
-    def iteration():
-        """one ADMM iteration enqueued on st.stream (the part of the loop below that has no host logic)"""
-        sm = st.stream
-        st.omega_step(upper)
-        Cq = st.W if latent else None
-        if upper:
-            _lib.check(lib.gg_prox_mgl_upper_batch(_p(st.Omega_new), _p(st.Omega), _p(st.X), _p(st.Theta),
-                                                   _p(st.ctrl), lam1_arg, lam2_arg, regi, mpp, p, nprob, _p(partials),
-                                                   sm), "gg_prox_mgl_upper")
-        elif big_K:
-            _lib.check(lib.gg_pack_bands(_p(st.Omega_new), _p(st.L), _p(st.X), _p(st.ctrl), M, p, 1, _p(vband), sm),
-                       "gg_pack_bands")
-            _lib.check(lib.gg_prox_band(_p(vband), _p(tband), _p(st.ctrl), lambda1, lambda2, regi, M, p, p, 0, sm),
-                       "gg_prox_band")
-            _lib.check(lib.gg_unpack_dual(_p(tband), _p(st.Omega_new), _p(st.Omega), _p(st.X), _p(st.Theta), _p(Cq),
-                                          _p(st.ctrl), M, p, 1, _p(partials), sm), "gg_unpack_dual")
-        elif kind == "mgl":
-            _lib.check(prox_mgl_fn(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(Cq),
-                                   _p(st.ctrl), lam1_arg, lam2_arg, regi, mpp, p, nprob, _p(partials), sm),
-                       "gg_prox_mgl")
-        elif Mblk is not None:
-            _lib.check(lib.gg_prox_fsgl(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(Cq),
-                                        _p(st.ctrl), float(lambda1), int(Mblk), M, p, _p(partials), _p(blk_nrm), sm),
-                       "gg_prox_fsgl")
-        else:
-            _lib.check(lib.gg_prox_sgl(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(Cq),
-                                       _p(st.ctrl), float(lambda1), _p(st.lam_mat), M, p, _p(partials), _p(st.pvec), sm),
-                       "gg_prox_sgl")
-        if latent:
-            st.l_step()
-            _lib.check(lib.gg_dual_update(_p(st.X), _p(st.Omega_new), _p(st.Omega), _p(st.Theta), _p(st.L),
-                                          _p(st.ctrl), M, p, mpp, 1 if kind == "sgl" else 0, _p(partials), sm),
-                       "gg_dual_update")
-        _lib.check(lib.gg_stop_update(_p(partials), nparts, _p(st.ctrl), _p(st.hist), st.hist_cap, _p(st.pdim),
-                                      tol, rtol, 1 if update_rho else 0, nprob, sm), "gg_stop_update")
-        st.swap()
-
-    if graph is None:
-        graph = p <= _env_int("GG_GRAPH_MAX_P", 640) and _env_int("GG_GRAPH", 0) != 0
-    use_graph = (graph and stopping_criterion == "boyd" and not measure and not verbose and trace is None
-                 and not _DEBUG_KEEP_INPUT and st.eig.nb2 == 0 and max_iter >= 4)
-    graph_done = False
-    first_eager = 0
-    if use_graph:
-        # lambdas are read from the control block by the MGL prox, so the key does not contain them for 'mgl'
-        key = (kind, regi, Mblk, latent, tol, rtol, update_rho, None if kind == "mgl" else float(lambda1), st.hist_cap)
-        it = 0
-        graphs = st._graphs.get(key)
-        if graphs is None:
-            iteration()                          # first iteration eagerly: every kernel module is loaded before capture
-            it = 1
-            graphs = [None, None]
-            cap = torch.cuda.Stream(device=st.dev)
-            cap.wait_stream(torch.cuda.current_stream())
-            keep = (st.stream, st.nswap, st.Omega, st.Omega_new)
-            try:
-                with _H2D_LOCK:                  # one capture at a time (torch's capture bookkeeping is process wide)
-                    for _ in range(2):
-                        par = st.nswap % 2
-                        g = torch.cuda.CUDAGraph()
-                        with torch.cuda.graph(g, stream=cap, capture_error_mode="thread_local"):
-                            st.stream = torch.cuda.current_stream().cuda_stream
-                            iteration()
-                        graphs[par] = g
-            except Exception as ex:              # capture not possible here: run the loop eagerly, say so once
-                if not _STAGE.get("graph_warned"):
-                    _STAGE["graph_warned"] = True
-                    import warnings
-                    warnings.warn(f"gglasso_b200: CUDA graph capture of the ADMM iteration failed ({type(ex).__name__}: "
-                                  f"{str(ex)[:120]}); running eagerly")
-                graphs = False
-            # two captures = two pointer swaps: the pointers are back where they were, nothing has run
-            st.stream, st.nswap, st.Omega, st.Omega_new = keep
-            torch.cuda.current_stream().wait_stream(cap)
-            st._graphs[key] = graphs
-        if graphs is False:
-            use_graph = False
-            first_eager = it
-        while use_graph and it < max_iter:
-            graphs[st.nswap % 2].replay()
-            st.swap()
-            it += 1
-            if it % check_every == 0 or it == max_iter:
-                if np.all(st.read_ctrl()[:, C_DONE] != 0):
-                    break
-        if use_graph:
-            it_done = it
-            graph_done = True
-
-    for it in range(max_iter if graph_done else first_eager, max_iter):
+    for it in range(max_iter):
         if measure:
             torch.cuda.synchronize()
             t0 = time.time()
@@ -653,37 +561,35 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
             beta = (st.nk if st.nk is not None else torch.ones(M, dtype=torch.float64, device=st.dev)) / st.ctrl[0, C_RHO]
             Dw = st.eig.D
             logdet_dev = torch.log(0.5 * (torch.sqrt(Dw * Dw + 4 * beta[:, None]) + Dw)).sum()
-        C = st.W if latent else None
+        Om, Om_prev, X, Th, ctl, parts = (_p(st.Omega_new), _p(st.Omega), _p(st.X), _p(st.Theta), _p(st.ctrl),
+                                           _p(partials))
         if upper:
-            _lib.check(lib.gg_prox_mgl_upper_batch(_p(st.Omega_new), _p(st.Omega), _p(st.X), _p(st.Theta),
-                                                   _p(st.ctrl), lam1_arg, lam2_arg, regi, mpp, p, nprob, _p(partials),
-                                                   stream), "gg_prox_mgl_upper")
+            _lib.check(lib.gg_prox_mgl_upper_batch(Om, Om_prev, X, Th, ctl, lam1_arg, lam2_arg, regi, mpp, p, nprob,
+                                                   parts, stream), "gg_prox_mgl_upper")
         elif big_K:
-            _lib.check(lib.gg_pack_bands(_p(st.Omega_new), _p(st.L), _p(st.X), _p(st.ctrl), M, p, 1, _p(vband), stream),
-                       "gg_pack_bands")
-            _lib.check(lib.gg_prox_band(_p(vband), _p(tband), _p(st.ctrl), lambda1, lambda2, regi, M, p, p, 0, stream),
+            _lib.check(lib.gg_pack_bands(Om, _p(st.L), X, ctl, M, p, 1, _p(vband), stream), "gg_pack_bands")
+            _lib.check(lib.gg_prox_band(_p(vband), _p(tband), ctl, lambda1, lambda2, regi, M, p, p, 0, stream),
                        "gg_prox_band")
-            _lib.check(lib.gg_unpack_dual(_p(tband), _p(st.Omega_new), _p(st.Omega), _p(st.X), _p(st.Theta), _p(C),
-                                          _p(st.ctrl), M, p, 1, _p(partials), stream), "gg_unpack_dual")
+            _lib.check(lib.gg_unpack_dual(_p(tband), Om, Om_prev, X, Th, _p(C), ctl, M, p, 1, parts, stream),
+                       "gg_unpack_dual")
+        elif ragged_mgl:
+            _lib.check(lib.gg_prox_mgl_ragged(Om, Om_prev, X, Th, ctl, lam1_arg, lam2_arg, regi, mpp, p, nprob,
+                                              _p(st.pvec), parts, stream), "gg_prox_mgl")
         elif kind == "mgl":
-            _lib.check(prox_mgl_fn(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(C),
-                                   _p(st.ctrl), lam1_arg, lam2_arg, regi, mpp, p, nprob, _p(partials), stream),
-                       "gg_prox_mgl")
+            _lib.check(lib.gg_prox_mgl_batch(Om, Om_prev, _p(st.L), X, Th, _p(C), ctl, lam1_arg, lam2_arg, regi, mpp,
+                                             p, nprob, parts, stream), "gg_prox_mgl")
         elif Mblk is not None:
-            _lib.check(lib.gg_prox_fsgl(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(C),
-                                        _p(st.ctrl), float(lambda1), int(Mblk), M, p, _p(partials), _p(blk_nrm),
-                                        stream), "gg_prox_fsgl")
+            _lib.check(lib.gg_prox_fsgl(Om, Om_prev, _p(st.L), X, Th, _p(C), ctl, float(lambda1), int(Mblk), M, p,
+                                        parts, _p(blk_nrm), stream), "gg_prox_fsgl")
         else:
-            _lib.check(lib.gg_prox_sgl(_p(st.Omega_new), _p(st.Omega), _p(st.L), _p(st.X), _p(st.Theta), _p(C),
-                                       _p(st.ctrl), float(lambda1), _p(st.lam_mat), M, p, _p(partials), _p(st.pvec),
-                                       stream), "gg_prox_sgl")
+            _lib.check(lib.gg_prox_sgl(Om, Om_prev, _p(st.L), X, Th, _p(C), ctl, float(lambda1), _p(st.lam_mat), M, p,
+                                       parts, _p(st.pvec), stream), "gg_prox_sgl")
         if _DEBUG_KEEP_INPUT:
             _debug_check(st, it, "after prox", Theta=st.Theta, X=st.X)
         if latent:
             st.l_step()
-            _lib.check(lib.gg_dual_update(_p(st.X), _p(st.Omega_new), _p(st.Omega), _p(st.Theta), _p(st.L),
-                                          _p(st.ctrl), M, p, mpp, 1 if kind == "sgl" else 0, _p(partials), stream),
-                       "gg_dual_update")
+            _lib.check(lib.gg_dual_update(X, Om, Om_prev, Th, _p(st.L), ctl, M, p, mpp, 1 if kind == "sgl" else 0,
+                                          parts, stream), "gg_dual_update")
         if measure:
             torch.cuda.synchronize()
             runtime[it] = time.time() - t0
@@ -691,19 +597,17 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
                 objective[it] = _objective(st, st.Omega_new, lambda1, lambda2, regi, logdet_dev)
         it_done = it + 1
         if stopping_criterion == "boyd":
-            _lib.check(lib.gg_stop_update(_p(partials), nparts, _p(st.ctrl), _p(st.hist), st.hist_cap, _p(st.pdim),
-                                          tol, rtol, 1 if update_rho else 0, nprob, stream), "gg_stop_update")
+            _lib.check(lib.gg_stop_update(parts, nparts, ctl, _p(st.hist), st.hist_cap, _p(st.pdim), tol, rtol,
+                                          1 if update_rho else 0, nprob, stream), "gg_stop_update")
             st.swap()
-            if trace is not None:       # test hook: per-iteration state (X before the rho rescale, like the oracle)
-                if st.ctrl[0, C_DONE].item() != 0 and st.ctrl[0, C_ITER].item() != it + 1:
-                    pass
-                elif callable(trace):
-                    if upper:
-                        st.mirror()
+            # test hook: per-iteration state (X before the rho rescale, like the oracle); iterations after the done flag
+            # are no-ops and are skipped
+            if trace is not None and not (st.ctrl[0, C_DONE].item() != 0 and st.ctrl[0, C_ITER].item() != it + 1):
+                if upper:
+                    st.mirror()
+                if callable(trace):
                     trace(st, it)
                 else:
-                    if upper:
-                        st.mirror()
                     trace.append(dict(Omega=st.Omega.cpu().numpy(), Theta=st.Theta.cpu().numpy(),
                                       L=None if st.L is None else st.L.cpu().numpy(), X=st.X.cpu().numpy()))
             if (it + 1) % check_every == 0 or it + 1 == max_iter:
@@ -745,20 +649,9 @@ def run_admm(kind, S, Omega_0, Theta_0, X_0, *, lambda1, lambda2=None, reg=None,
         hist = st.hist.cpu().numpy()
         info["iters"] = iters
         info["hist"] = hist
-        statuses = []
-        for q in range(nprob):
-            n = iters[q]
-            r, s, e_pri, e_dual = hist[q, n - 1, :4]
-            if ctrl[q, C_DONE] != 0:
-                statuses.append("optimal")
-            elif r <= e_pri:
-                statuses.append("primal optimal")
-            elif s <= e_dual:
-                statuses.append("dual optimal")
-            else:
-                statuses.append("max iterations reached")
-        info["status"] = statuses
-        info["residual"] = [np.maximum(hist[q, :iters[q], 0], hist[q, :iters[q], 1]) for q in range(nprob)]
+        per_problem = [boyd_status(ctrl[q], hist[q]) for q in range(nprob)]
+        info["status"] = [status for status, _ in per_problem]
+        info["residual"] = [residual for _, residual in per_problem]
     else:
         info["iters"] = np.full(nprob, it_done)
         info["status"] = [status if status else "max iterations reached"] * nprob
@@ -790,9 +683,7 @@ def _kkt_residual(kind, st, lambda1, lambda2, regi, latent):
     """
     lib, stream = st.lib, st.stream
     M, p = st.M, st.p
-    ctrl1 = torch.zeros((st.nprob, CTRL_STRIDE), dtype=torch.float64, device=st.dev)
-    ctrl1[:, C_RHO] = 1.0
-    ctrl1[:, 1] = 1.0
+    ctrl1 = torch.from_numpy(control_block(st.nprob, 1.0)).to(st.dev, non_blocking=True)
     rho = st.ctrl[:, C_RHO].reshape(-1, 1, 1).repeat_interleave(st.mpp, 0)
     Xu = rho * st.X                                     # unscaled dual
     Omega, Theta = st.Omega, st.Theta

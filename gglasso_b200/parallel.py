@@ -188,7 +188,7 @@ def run_admm_mgl_dist(S_local, lambda1, lambda2, reg, Omega_0_local, K_total=Non
                       verbose=False, latent=False, mu1_local=None, group=None, check_every=1):
     """device loop of ADMM_MGL_dist; returns (AdmmState, info) without copying the solution to the host."""
     from . import _lib
-    from ._engine import AdmmState, _p
+    from ._engine import AdmmState, _p, boyd_status
     from ._lib import C_DONE, C_ITER, C_STATUS, NPART
     assert reg in ['GGL', 'FGL'] and min(lambda1, lambda2) > 0 and rho > 0
     K_loc, p, _ = S_local.shape
@@ -279,17 +279,8 @@ def run_admm_mgl_dist(S_local, lambda1, lambda2, reg, Omega_0_local, K_total=Non
         raise _lib.GGLassoB200Error(f"non-finite residual after {int(ctrl[0, C_ITER])} iteration(s): the input is not "
                                     "finite or an eigendecomposition broke down")
     n = int(ctrl[0, C_ITER])
-    hist = st.hist[0, :n].cpu().numpy()
-    r, s, e_pri, e_dual = hist[n - 1, :4]
-    if ctrl[0, C_DONE] != 0:
-        status = "optimal"
-    elif r <= e_pri:
-        status = "primal optimal"
-    elif s <= e_dual:
-        status = "dual optimal"
-    else:
-        status = "max iterations reached"
-    info = {"status": status, "iterations": n, "residual": np.maximum(hist[:, 0], hist[:, 1])}
+    status, residual = boyd_status(ctrl[0], st.hist[0, :n].cpu().numpy())
+    info = {"status": status, "iterations": n, "residual": residual}
     return st, info
 
 
@@ -360,7 +351,7 @@ def _score_device(st, Omega_unused, N, gamma, method):
     reductions over arrays that are already resident."""
     K, p = st.M, st.p
     Theta = st.Theta
-    D = st.eig.eigh(Theta.clone(), ctrl=None, mpp=1, vectors=0, stream=st.stream)          # (K,p)
+    D = st.eigvalsh(Theta)          # (K,p)
     dmin = D.min(dim=1).values
     logdet = torch.where(dmin > 1e-12, torch.log(D.clamp_min(1e-300)).sum(1), torch.full_like(dmin, -float("inf")))
     inner = (st.S * Theta).sum((1, 2))
@@ -404,7 +395,7 @@ def grid_search_device(S, N, reg, l1, l2, method="eBIC", gamma=0.1, tol=1e-7, rt
     def run_columns(cols, out):
         """one worker = one CUDA stream: its columns run back to back, warm starts stay on the device"""
         b, b_score, b_ix = None, np.inf, None
-        st = None                                 # one state per worker: buffers, workspace and iteration graphs are reused
+        st = None                                 # one state per worker: buffers and workspace are reused
         for g2 in cols:
             Omega_0 = eye
             for g1 in range(len(l2)):

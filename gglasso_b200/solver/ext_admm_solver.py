@@ -15,7 +15,7 @@ import numpy as np
 import torch
 
 from .. import _lib
-from .._engine import AdmmState, _p, to_dev, to_host
+from .._engine import AdmmState, _p, boyd_status, control_block, to_dev, to_host
 from .._lib import C_DONE, C_ITER, NPART
 
 
@@ -170,17 +170,7 @@ def ext_ADMM_MGL(S: dict,
     ctrl = st.read_ctrl()
     if stopping_criterion == 'boyd':
         n_it = int(ctrl[0, C_ITER])
-        hist = st.hist[0, :n_it].cpu().numpy()
-        r_t, s_t, e_pri, e_dual = hist[n_it - 1, :4]
-        if ctrl[0, C_DONE] != 0:
-            status = 'optimal'
-        elif r_t <= e_pri:
-            status = 'primal optimal'
-        elif s_t <= e_dual:
-            status = 'dual optimal'
-        else:
-            status = 'max iterations reached'
-        residual = np.maximum(hist[:, 0], hist[:, 1])
+        status, residual = boyd_status(ctrl[0], st.hist[0, :n_it].cpu().numpy())
     else:
         n_it = it_done
         if status != 'optimal':
@@ -192,8 +182,8 @@ def ext_ADMM_MGL(S: dict,
     Om, Th, X0h, X1h = to_host(Omega_d), to_host(st.Theta), to_host(st.X), to_host(X1d)
     Lh = to_host(st.L) if latent else np.zeros((K, pm, pm))
     TL = st.Theta - st.L if latent else st.Theta
-    D = st.eig.eigh(TL.clone(), ctrl=None, mpp=1, vectors=0, stream=stream).cpu().numpy()
-    DL = st.eig.eigh(st.L.clone(), ctrl=None, mpp=1, vectors=0, stream=stream).cpu().numpy() if latent else None
+    D = st.eigvalsh(TL).cpu().numpy()
+    DL = st.eigvalsh(st.L).cpu().numpy() if latent else None
     sol = {'Omega': {}, 'Theta': {}, 'L': {}, 'X0': {}, 'X1': {}}
     for k in range(K):
         n = p[k]
@@ -219,16 +209,14 @@ def ext_ADMM_MGL(S: dict,
 def _kkt(st, Lam, X1d, Gd, Lg, lam1, lambda2, latent, mask, lib, stream):
     """KKT residual of the non-conforming problem (ext_admm_solver.py:349-392).  prox / eigendecompositions run
     through the CUDA kernels; norms and differences of resident arrays are torch glue on the device."""
-    from .._lib import CTRL_STRIDE, C_RHO
+    from .._lib import C_RHO
     K, pm = st.M, st.p
     dev = st.dev
     rho = st.ctrl[0, C_RHO]
     Omega, Theta = st.Omega, st.Theta
     L = st.L if latent else torch.zeros_like(Theta)
     X0u, X1u = rho * st.X, rho * X1d
-    ctrl1 = torch.zeros((1, CTRL_STRIDE), dtype=torch.float64, device=dev)
-    ctrl1[:, C_RHO] = 1.0
-    ctrl1[:, 1] = 1.0
+    ctrl1 = torch.from_numpy(control_block(1, 1.0)).to(dev, non_blocking=True)
 
     def nrm(A):
         return torch.sqrt(((A * mask) ** 2).sum((1, 2)))

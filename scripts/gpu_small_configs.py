@@ -1,4 +1,4 @@
-"""cfg1 / cfg2 / cfg4 timings on the GPU with and without CUDA-graph iterations, and the real reference on the host cores.
+"""cfg1 / cfg2 / cfg4 timings on the GPU, and the real reference on the host cores.
 usage: python scripts/gpu_small_configs.py [out.json]"""
 import contextlib, io, json, os, sys, time
 import numpy as np
@@ -37,24 +37,21 @@ cases = {
 }
 for name, (gpu, cpu) in cases.items():
     rec = {}
-    for g in (0, 1):
-        os.environ["GG_GRAPH"] = str(g)
-        gpu()
-        rec[f"gpu_graph{g}_s"], (sol, info) = wall(gpu)
+    gpu()
+    rec["gpu_s"], (sol, info) = wall(gpu)
     cpu()
     rec["cpu_reference_s"], (rsol, rinfo) = wall(cpu, reps=2)
     rec["theta_rel_err"] = float(np.linalg.norm(sol["Theta"] - rsol["Theta"]) / np.linalg.norm(rsol["Theta"]))
-    rec["speedup_graph1"] = rec["cpu_reference_s"] / rec["gpu_graph1_s"]
+    rec["speedup"] = rec["cpu_reference_s"] / rec["gpu_s"]
     print(name, rec, flush=True)
     out[name] = rec
 
 S4 = ref_inputs.load("cfg4"); N4 = np.full(10, 1000)
 l1, l2 = np.logspace(0, -3, 10), np.logspace(-1, -4, 10)
-for g, ns in ((0, 5), (1, 5), (1, 10), (1, 3), (1, 1)):
-    os.environ["GG_GRAPH"] = str(g)
+for ns in (5, 10, 3, 1):
     grid_search_device(S4, N4, "GGL", l1[4:5], l2[:2], gamma=0.1, tol=1e-5, rtol=1e-5)
     t, (scores, iters, ix, best) = wall(lambda: grid_search_device(S4, N4, "GGL", l1, l2, gamma=0.1, tol=1e-7, rtol=1e-7, n_streams=ns), reps=1)
-    rec = {"graph": g, "n_streams": ns, "seconds": t, "iterations": int(iters.sum()), "best": [int(i) for i in ix]}
+    rec = {"n_streams": ns, "seconds": t, "iterations": int(iters.sum()), "best": [int(i) for i in ix]}
     print("cfg4_grid", rec, flush=True)
-    out[f"cfg4_grid_graph{g}_streams{ns}"] = rec
+    out[f"cfg4_grid_streams{ns}"] = rec
 json.dump(out, open(sys.argv[1] if len(sys.argv) > 1 else "gpurun_out/small_configs.json", "w"), indent=1)
